@@ -2,7 +2,7 @@
 """Benchmark of the GNNAE train step (BASELINE.json: jets/sec, fwd+bwd+Adam, Chamfer loss, N=30).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--num-nodes 30|150]
-                    [--batch B] [--precision bf16|fp32]
+                    [--batch B] [--precision bf16|fp32] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  Headline workload: reference CLI-default architecture, synthetic JetNet-shaped
 jets, 4096 jets per GPU (BASELINE config 2 at N=1; 8 GPUs = config 4's 32768-jet global batch), weak scaling.
@@ -15,6 +15,8 @@ at --gpus G > 1 also "dp_parity" (parameters bit-identical across ranks, G-rank 
 ranks); "e2e" goes through the public ``GNNAETrainer.step`` with a pinned host batch per step and a
 device->host read of the loss.  ``--impl reference`` times the CPU PyTorch restatement of the reference's
 train step (oracle/torch_port.py, "port") on the host cores.
+``--dump-outputs DIR`` also writes what the last timed step computed as DIR/<name>.npy (``dump_timed_outputs``); inputs and
+initial parameters are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -330,6 +332,30 @@ def _dp_parity(dev, world, rank, precision):
     dist.barrier()
     return err
 
+
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_timed_outputs(tr, out_dir, limit=DUMP_LIMIT_BYTES):
+    """Write what the last timed step (compute_gradients + apply_gradients) hands a caller to ``out_dir``/<name>.npy:
+    latent (B, latent) and recon (B, N, F) of its forward pass, loss (float64, the value ``GNNAETrainer.step`` returns), grad
+    (the flat parameter gradient) and params (the flat parameters after the optimiser update), all float32 but the loss.
+    Above ``limit`` bytes in all, latent and recon keep a fixed sample of jets: the sorted rows
+    ``numpy.random.default_rng(0).choice(B, k, replace=False)``, the same for every build at the same arguments."""
+    import numpy as np
+    out = {"latent": tr.latent, "recon": tr.recon, "grad": tr.grad, "params": tr.flat}
+    out = {k: v.detach().cpu().numpy().astype(np.float32, copy=False) for k, v in out.items()}
+    out["loss"] = np.float64(tr.loss_from_stats(tr.stats.cpu()))
+    per_jet = out["latent"][0].nbytes + out["recon"][0].nbytes
+    fixed = out["grad"].nbytes + out["params"].nbytes + 8 + 128 * len(out)      # + the .npy headers
+    k = min(tr.B, (limit - fixed) // per_jet)
+    if k < tr.B:
+        rows = np.sort(np.random.default_rng(0).choice(tr.B, k, replace=False))
+        out["latent"], out["recon"] = out["latent"][rows], out["recon"][rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
 # --------------------------------------------------------------------------------------------------
 # our arm
 # --------------------------------------------------------------------------------------------------
@@ -409,6 +435,8 @@ def run_ours(args):
         tr.apply_gradients()
         e.record()
     barrier()
+    if args.dump_outputs and rank == 0:      # before the e2e loop below moves the parameters on
+        dump_timed_outputs(tr, args.dump_outputs)
     launches = ops.LAUNCHES["count"] - launches0
     ms_total = rank_max(sum(s.elapsed_time(e) for s, e in ev))
     ms_step = ms_total / args.steps
@@ -604,7 +632,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the extra BASELINE configurations of the 'configs' object")
     ap.add_argument("--cpu-sample", type=int, default=0, help="jets per CPU-baseline step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -305,3 +305,33 @@ def test_bench_reference_arm_prints_one_json_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["gpu_launches"] == 0
+
+
+def test_bench_dump_writes_the_step_outputs_within_the_limit(tmp_path):
+    """`bench.py --dump-outputs`: one float32 / float64 .npy per output of the step; above the byte limit latent and recon keep the
+    same seeded sample of jets on every call, and the files stay within the limit."""
+    import types
+    import numpy as np
+    import torch
+    import bench
+    B, N = 50, 7
+    g = torch.Generator().manual_seed(0)
+    tr = types.SimpleNamespace(B=B, latent=torch.randn(B, 4, generator=g), recon=torch.randn(B, N, 3, generator=g),
+                               grad=torch.randn(100, generator=g), flat=torch.randn(100, generator=g),
+                               stats=torch.tensor([0, 0, 2.5, 0, 0, 0, 0, 0]), loss_from_stats=lambda s: float(s[2]))
+    load = lambda d: {p.stem: np.load(p) for p in d.glob("*.npy")}
+    bench.dump_timed_outputs(tr, str(tmp_path / "all"))
+    full = load(tmp_path / "all")
+    assert sorted(full) == ["grad", "latent", "loss", "params", "recon"]
+    assert all(a.dtype in (np.float32, np.float64) for a in full.values()) and full["loss"] == 2.5
+    for k, t in (("latent", tr.latent), ("recon", tr.recon), ("grad", tr.grad), ("params", tr.flat)):
+        assert np.array_equal(full[k], t.numpy())
+    limit = 2 * 100 * 4 + 8 + 5 * 128 + 20 * (4 + N * 3) * 4      # room for 20 of the 50 jets
+    for d in ("a", "b"):
+        bench.dump_timed_outputs(tr, str(tmp_path / d), limit=limit)
+        assert sum(p.stat().st_size for p in (tmp_path / d).glob("*.npy")) <= limit
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    rows = np.sort(np.random.default_rng(0).choice(B, 20, replace=False))
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    assert np.array_equal(a["recon"], full["recon"][rows]) and np.array_equal(a["latent"], full["latent"][rows])
+    assert np.array_equal(a["grad"], full["grad"]) and np.array_equal(a["params"], full["params"])
