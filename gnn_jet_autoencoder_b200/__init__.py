@@ -7,9 +7,10 @@ of ``libgnnjet_b200.so`` (C-ABI: include/gnnjet_b200.h); there is no CPU or eage
 """
 from . import _lib
 from .models import GraphNet, Encoder, Decoder
-from .losses import ChamferLoss, HungarianMSELoss
+from .losses import ChamferLoss, EMDLoss, HungarianMSELoss
 from .trainer import GNNAETrainer, synthetic_jets
 from . import anomaly
 from .permutation import PermutationTest
 
-__all__ = ["GraphNet", "Encoder", "Decoder", "ChamferLoss", "HungarianMSELoss", "GNNAETrainer", "synthetic_jets", "anomaly", "PermutationTest", "_lib"]
+__all__ = ["GraphNet", "Encoder", "Decoder", "ChamferLoss", "EMDLoss", "HungarianMSELoss", "GNNAETrainer", "synthetic_jets", "anomaly",
+           "PermutationTest", "_lib"]

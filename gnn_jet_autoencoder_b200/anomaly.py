@@ -1,5 +1,6 @@
 """Anomaly-score distances of reference utils/jet_analysis/anomaly_detection.py (:454-510) on one kernel launch:
-``mse``, ``chamfer`` (Euclidean norm) and ``chamfer_lorentz`` with the reference's signatures and return shapes.
+``mse``, ``chamfer`` (Euclidean norm) and ``chamfer_lorentz`` with the reference's signatures and return shapes, the
+optimal-matching scores ``hungarian`` / ``hungarian_lorentz``, and the exact energy mover's distance ``emd``.
 
 The reference builds the (B, N, N, D) difference tensor and, in the batched form, goes through a DataLoader with one
 host <-> device round trip per batch (:471-481); here a CTA per jet keeps the two particle sets in shared memory and
@@ -98,3 +99,72 @@ def hungarian(p: torch.Tensor, q: torch.Tensor, batch_size: int = -1) -> torch.T
 def hungarian_lorentz(p: torch.Tensor, q: torch.Tensor, batch_size: int = -1) -> torch.Tensor:
     """anomaly_detection.py:550-590: the same with the Lorentz norm squared of the differences as the matching cost."""
     return _batched(lambda a, b: _hungarian(a, b, True), p, q, batch_size)
+
+
+def _emd_polar(x: torch.Tensor, polar_coord: bool) -> torch.Tensor:
+    """[pt, eta, phi] jets as ``gj_emd`` takes them: as given, or converted from Cartesian 3- / 4-vectors like
+    ``losses.hungarian_preprocess`` does."""
+    from .losses import _to_polar
+    if x.dim() != 3:
+        raise ValueError(f"expected (B, N, D) jets, got {tuple(x.shape)}")
+    if polar_coord:
+        if x.shape[-1] != 3:
+            raise ValueError(f"polar_coord=True expects [pt, eta, phi] jets (B, N, 3), got {tuple(x.shape)}")
+        return x
+    return _to_polar(x)
+
+
+def _emd_solve(p: torch.Tensor, q: torch.Tensor, R: float, beta: float, norm: bool, periodic_phi: bool, want_flow: bool = False,
+               want_grad: bool = False, want_potentials: bool = False):
+    """One ``gj_emd`` launch on [pt, eta, phi] jets p (B, Np, 3), q (B, Nq, 3): (emd (B,) float64, flow (B, Np, Nq) float64,
+    dEMD/dp (B, Np, 3) float32, potentials (B, Np+1+Nq+1) float64), the last three None unless asked for.  Raises if a jet's
+    solver did not converge."""
+    if p.dim() != 3 or q.dim() != 3 or p.shape[0] != q.shape[0] or p.shape[2] != 3 or q.shape[2] != 3:
+        raise ValueError(f"expected (B, Np, 3) and (B, Nq, 3) jets, got {tuple(p.shape)} and {tuple(q.shape)}")
+    dev = p.device if p.is_cuda else _device()
+    pc = p.detach().to(device=dev, dtype=torch.float32).contiguous()
+    qc = q.detach().to(device=dev, dtype=torch.float32).contiguous()
+    B, Np, Nq = pc.shape[0], pc.shape[1], qc.shape[1]
+    f64 = dict(device=dev, dtype=torch.float64)
+    emd = torch.empty((B,), **f64)
+    flow = torch.empty((B, Np, Nq), **f64) if want_flow else None
+    dp = torch.empty((B, Np, 3), device=dev, dtype=torch.float32) if want_grad else None
+    pot = torch.empty((B, Np + Nq + 2), **f64) if want_potentials else None
+    status = torch.empty((B,), device=dev, dtype=torch.int32)
+    flags = (_lib.GJ_EMD_NORM if norm else 0) | (_lib.GJ_EMD_PERIODIC_PHI if periodic_phi else 0)
+    ptr = lambda t: t.data_ptr() if t is not None else None
+    with torch.cuda.device(dev):
+        _lib.check(_lib.load().gj_emd(B, Np, Nq, pc.data_ptr(), qc.data_ptr(), float(R), float(beta), flags, emd.data_ptr(), ptr(flow),
+                                      ptr(dp), ptr(pot), status.data_ptr(), None, 0, torch.cuda.current_stream().cuda_stream), "gj_emd")
+    bad = int((status != 0).sum())
+    if bad:
+        raise RuntimeError(f"gj_emd: the transport solver did not converge for {bad} of {B} jets")
+    return emd, flow, dp, pot
+
+
+def emd(p: torch.Tensor, q: torch.Tensor, R: float = 1.0, beta: float = 1.0, norm: bool = False, periodic_phi: bool = False,
+        polar_coord: bool = True, batch_size: int = -1, return_flow: bool = False):
+    """Exact energy mover's distance per jet (energyflow.emd.emd's definition; the EMD score of anomaly_detection.py), solved for
+    the whole batch in one launch: (B,) float64 tensor of
+
+        EMD = min_f sum_ij f_ij (theta_ij / R)^beta + |W_p - W_q|,  sum_j f_ij <= w_i, sum_i f_ij <= w'_j, sum f = min(W_p, W_q)
+
+    with weights w = max(pt, 0) and theta_ij = sqrt(deta^2 + dphi^2) (dphi wrapped into [-pi, pi) with ``periodic_phi``).
+    p (B, Np, 3) and q (B, Nq, 3) are [pt, eta, phi] jets, or Cartesian 3- / 4-vectors with ``polar_coord=False``; Np and Nq
+    may differ (at most 150 each).  ``norm`` divides each jet's weights by its total.  ``return_flow`` also returns the optimal
+    flow (B, Np, Nq) float64.  A positive ``batch_size`` walks the jets in batches and returns CPU tensors, like the other
+    scores here.  Raises if a jet's solver did not converge."""
+    def one(a, b):
+        dev = a.device if a.is_cuda else _device()
+        e, f, _, _ = _emd_solve(_emd_polar(a.to(dev), polar_coord), _emd_polar(b.to(dev), polar_coord), R, beta, norm, periodic_phi,
+                                want_flow=return_flow)
+        return e, f
+    if batch_size is not None and batch_size > 0 and p.shape[0] > 0:
+        parts = [one(p[i:i + batch_size], q[i:i + batch_size]) for i in range(0, p.shape[0], batch_size)]
+        e = torch.cat([x[0].cpu() for x in parts])
+        f = torch.cat([x[1].cpu() for x in parts]) if return_flow else None
+    else:
+        e, f = one(p, q)
+        if not p.is_cuda:
+            e, f = e.cpu(), (f.cpu() if return_flow else None)
+    return (e, f) if return_flow else e

@@ -107,6 +107,8 @@ void gj_tc_plan_info(MPLayout, int*);
 int gj_chamfer_launch(int, int, int, int, int, float, float, const float*, const float*, float*, float*, float*, cudaStream_t);
 int gj_pair_min_dist_launch(int, int, int, int, int, const float*, const float*, float*, float*, cudaStream_t);
 int gj_assignment_launch(int, int, int, int, const float*, const float*, int*, float*, cudaStream_t);
+int gj_emd_check(int, int, int, float, float, int);
+int gj_emd_launch(int, int, int, const float*, const float*, float, float, int, double*, double*, float*, double*, int*, cudaStream_t);
 int gj_linear_fwd_launch(int, int, int, const float*, const float*, const float*, float*, cudaStream_t);
 size_t gj_linear_bwd_ws_bytes(int, int, int);
 int gj_linear_bwd_launch(int, int, int, const float*, const float*, const float*, float*, float*, float*, void*, size_t, cudaStream_t);
@@ -489,6 +491,17 @@ int gj_assignment(int32_t batch, int32_t n, int32_t dim, int32_t lorentz, const 
   g_err[0] = 0;
   if (batch > 0 && (!p || !q || !col_for_row)) { gj_set_error("gj_assignment: null pointer"); return GJ_ERR_INVALID; }
   return gj_assignment_launch(batch, n, dim, lorentz, p, q, col_for_row, total_cost, (cudaStream_t)stream);
+}
+
+// the solver keeps its whole state in shared memory
+size_t gj_emd_workspace(int32_t, int32_t, int32_t) { return 0; }
+
+int gj_emd(int32_t batch, int32_t np_, int32_t nq, const float* p, const float* q, float R, float beta, int32_t flags, double* emd_out,
+           double* flow_out, float* dp_out, double* potentials_out, int32_t* status_out, void*, size_t, void* stream) {
+  g_err[0] = 0;
+  if (int rc = gj_emd_check(batch, np_, nq, R, beta, flags)) return rc;
+  if (batch > 0 && (!p || !q || !emd_out)) { gj_set_error("gj_emd: null pointer"); return GJ_ERR_INVALID; }
+  return gj_emd_launch(batch, np_, nq, p, q, R, beta, flags, emd_out, flow_out, dp_out, potentials_out, status_out, (cudaStream_t)stream);
 }
 
 int gj_linear_fwd(int32_t rows, int32_t in_f, int32_t out_f, const float* x, const float* w, const float* b, float* y,

@@ -1,4 +1,5 @@
-"""ChamferLoss: drop-in for reference utils/losses/chamfer_loss/chamfer_loss.py on one fused kernel."""
+"""ChamferLoss: drop-in for reference utils/losses/chamfer_loss/chamfer_loss.py on one fused kernel; HungarianMSELoss
+(utils/losses/hungarian_mse) with the matching on the device; EMDLoss, the exact energy mover's distance."""
 from __future__ import annotations
 
 import torch
@@ -105,3 +106,52 @@ class HungarianMSELoss(nn.Module):
         match = match.to(recons.device)
         recons_shuffle = torch.gather(recons, 1, match.unsqueeze(-1).expand(-1, -1, recons.shape[-1]))
         return nn.functional.mse_loss(recons_shuffle, target)
+
+
+class _EMD(torch.autograd.Function):
+    """Per-jet EMD (float64) of [pt, eta, phi] jets; backward returns the kernel's dEMD/dp, scaled per jet."""
+
+    @staticmethod
+    def forward(ctx, p, q, R, beta, norm, periodic_phi):
+        from .anomaly import _emd_solve
+        e, _, dp, _ = _emd_solve(p, q, R, beta, norm, periodic_phi, want_grad=ctx.needs_input_grad[0])
+        ctx.save_for_backward(dp)
+        ctx.p_meta = (p.dtype, p.device)
+        return e
+
+    @staticmethod
+    def backward(ctx, g):
+        dp, = ctx.saved_tensors
+        dtype, device = ctx.p_meta
+        return (dp.double() * g.to(dp.device, torch.float64)[:, None, None]).to(device=device, dtype=dtype), None, None, None, None, None
+
+
+class EMDLoss(nn.Module):
+    """Exact energy mover's distance between reconstructed and target jets (the loss reference utils/losses/emd_loss.py builds
+    from jetnet.losses.EMDLoss), solved on the device for the whole batch: ``anomaly.emd`` per jet, reduced by ``reduction``
+    ("sum" over jets, as ``ChamferLoss`` sums; "mean"; "none" for the (B,) vector).  recons (B, Np, D) receives the gradient,
+    target (B, Nq, D) does not; D = 3 ([pt, eta, phi]) or, with ``polar_coord=False``, Cartesian 3- / 4-vectors converted by the
+    differentiable ``_to_polar``.  Particle weights are max(pt, 0): a reconstructed particle with pt <= 0 gets no pt gradient."""
+
+    def __init__(self, R: float = 1.0, beta: float = 1.0, norm: bool = False, periodic_phi: bool = False, polar_coord: bool = True,
+                 reduction: str = "sum"):
+        super().__init__()
+        if reduction not in ("sum", "mean", "none"):
+            raise ValueError("reduction must be 'sum', 'mean' or 'none'")
+        if not (R > 0 and beta > 0):
+            raise ValueError(f"R and beta must be positive, got R={R}, beta={beta}")
+        self.R, self.beta, self.norm, self.periodic_phi = float(R), float(beta), bool(norm), bool(periodic_phi)
+        self.polar_coord, self.reduction = bool(polar_coord), reduction
+
+    def forward(self, recons: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
+        from .anomaly import _emd_polar
+        if target.requires_grad:
+            raise NotImplementedError("the EMD kernel differentiates w.r.t. the reconstruction only")
+        p = _emd_polar(recons, self.polar_coord)
+        q = _emd_polar(target.to(recons.device), self.polar_coord)
+        e = _EMD.apply(p, q, self.R, self.beta, self.norm, self.periodic_phi)
+        if self.reduction == "sum":
+            e = e.sum()
+        elif self.reduction == "mean":
+            e = e.mean()
+        return e.to(recons.dtype)

@@ -177,6 +177,34 @@ int gj_pair_min_dist(int32_t batch, int32_t np_, int32_t nq, int32_t dim, int32_
 int gj_assignment(int32_t batch, int32_t n, int32_t dim, int32_t lorentz, const float* p, const float* q,
                   int32_t* col_for_row, float* total_cost, void* stream);
 
+/* Exact energy mover's distance per jet, as energyflow.emd.emd defines it (Komiske, Metodiev, Thaler, PRL 123, 041801): the
+ * EMD scores of utils/jet_analysis/anomaly_detection.py (through energyflow) and the loss of utils/losses/emd_loss.py (through
+ * jetnet.losses.EMDLoss), both computed jet by jet on the host there.
+ * p (B,Np,3), q (B,Nq,3) as [pt, eta, phi]; weights w = max(pt, 0); theta_ij = sqrt(deta^2 + dphi^2) (dphi wrapped into
+ * [-pi, pi) with GJ_EMD_PERIODIC_PHI);
+ *   EMD = min_{f >= 0} sum_ij f_ij (theta_ij / R)^beta + |W_p - W_q|,
+ *         sum_j f_ij <= w_i, sum_i f_ij <= w'_j, sum_ij f_ij = min(W_p, W_q)        (W: total weight of a jet).
+ * GJ_EMD_NORM divides each non-empty jet's weights by its total (no imbalance term; an empty jet against a non-empty one gives 1).
+ * The problem is solved exactly as a balanced transportation problem with a dummy row (index Np, weight max(W_q - W_p, 0)) and a
+ * dummy column (index Nq, weight max(W_p - W_q, 0)) at cost 1 to every particle and 0 to each other; one CTA per jet, successive
+ * shortest paths with fp64 potentials and flows.  1 <= Np, Nq <= 150, R > 0, beta > 0.
+ * emd_out (B) fp64.  Optional (NULL = not written):
+ *   flow_out (B,Np,Nq) fp64: the optimal flow between the real particles (with GJ_EMD_NORM in normalised units);
+ *   dp_out (B,Np,3) fp32: gradient of emd_out w.r.t. p -- d/d(eta, phi) = sum_j f_ij beta theta_ij^(beta-2) / R^beta (deta, dphi)
+ *     (0 at theta = 0); d/dpt = the row's dual minus the dual of the dummy that absorbs the change (chain rule of the
+ *     normalisation with GJ_EMD_NORM), 0 where pt <= 0;
+ *   potentials_out (B, Np+1+Nq+1) fp64: optimal duals (u_0..u_Np, v_0..v_Nq) of the balanced problem, u_i + v_j <= c_ij with
+ *     equality where flow moves, and sum_i a_i u_i + sum_j b_j v_j = EMD;
+ *   status_out (B) int32: 0 converged, 1 augmentation cap N1 N2 + 4 (N1 + N2) + 64 reached, N1 = Np + 1, N2 = Nq + 1
+ *     (emd_out is then not optimal).
+ * gj_emd_workspace returns 0 for every shape (the solver's state lives in shared memory): workspace may be NULL. */
+#define GJ_EMD_NORM 1
+#define GJ_EMD_PERIODIC_PHI 2
+size_t gj_emd_workspace(int32_t batch, int32_t np_, int32_t nq);
+int gj_emd(int32_t batch, int32_t np_, int32_t nq, const float* p, const float* q, float R, float beta, int32_t flags,
+           double* emd_out, double* flow_out, float* dp_out, double* potentials_out, int32_t* status_out,
+           void* workspace, size_t workspace_bytes, void* stream);
+
 /* Flat fused Adam (torch.optim.Adam defaults: no weight decay, no amsgrad) over n floats.
  * grad_scale multiplies the incoming gradient, l1_lambda*sign(p) and 2*l2_lambda*p are added to it
  * (utils/train.py:376-384).  step is the 1-based step count of this update. */
