@@ -109,6 +109,9 @@ int gj_pair_min_dist_launch(int, int, int, int, int, const float*, const float*,
 int gj_assignment_launch(int, int, int, int, const float*, const float*, int*, float*, cudaStream_t);
 int gj_emd_check(int, int, int, float, float, int);
 int gj_emd_launch(int, int, int, const float*, const float*, float, float, int, double*, double*, float*, double*, int*, cudaStream_t);
+size_t gj_emd_loss_ws_bytes(int);
+int gj_emd_loss_check(int, int, int, int, float, float, int, size_t);
+int gj_emd_loss_launch(int, int, int, int, const float*, const float*, float, float, int, float, float*, float*, float*, void*, cudaStream_t);
 int gj_linear_fwd_launch(int, int, int, const float*, const float*, const float*, float*, cudaStream_t);
 size_t gj_linear_bwd_ws_bytes(int, int, int);
 int gj_linear_bwd_launch(int, int, int, const float*, const float*, const float*, float*, float*, float*, void*, size_t, cudaStream_t);
@@ -502,6 +505,17 @@ int gj_emd(int32_t batch, int32_t np_, int32_t nq, const float* p, const float* 
   if (int rc = gj_emd_check(batch, np_, nq, R, beta, flags)) return rc;
   if (batch > 0 && (!p || !q || !emd_out)) { gj_set_error("gj_emd: null pointer"); return GJ_ERR_INVALID; }
   return gj_emd_launch(batch, np_, nq, p, q, R, beta, flags, emd_out, flow_out, dp_out, potentials_out, status_out, (cudaStream_t)stream);
+}
+
+size_t gj_emd_loss_workspace(int32_t batch, int32_t) { return gj_emd_loss_ws_bytes(batch); }
+
+int gj_emd_loss(int32_t batch, int32_t n, int32_t dim, int32_t coords, const float* p, const float* q, float R, float beta,
+                int32_t flags, float scale, float* terms, float* failed, float* dp, void* workspace, size_t workspace_bytes,
+                void* stream) {
+  g_err[0] = 0;
+  if (int rc = gj_emd_loss_check(batch, n, dim, coords, R, beta, flags, workspace_bytes)) return rc;
+  if (!terms || !failed || (batch > 0 && (!p || !q || !workspace))) { gj_set_error("gj_emd_loss: null pointer"); return GJ_ERR_INVALID; }
+  return gj_emd_loss_launch(batch, n, dim, coords, p, q, R, beta, flags, scale, terms, failed, dp, workspace, (cudaStream_t)stream);
 }
 
 int gj_linear_fwd(int32_t rows, int32_t in_f, int32_t out_f, const float* x, const float* w, const float* b, float* y,

@@ -1,4 +1,4 @@
-"""The batch body of reference utils/train.py:51-85 (encoder -> decoder -> Chamfer (+L1/L2) -> backward ->
+"""The batch body of reference utils/train.py:51-85 (encoder -> decoder -> Chamfer / MSE / EMD (+L1/L2) -> backward ->
 two Adams) as a fixed sequence of fused kernels over flat buffers.
 
 * all parameters of encoder and decoder live in ONE flat fp32 buffer (the nn.Linear parameters are
@@ -21,7 +21,7 @@ import numpy as np
 import torch
 
 from . import _lib, ops
-from .losses import _norm_id
+from .losses import EMDLoss, _norm_id
 from .models.const import GLOBAL_MIX, LOCAL_MIX
 
 POLAR_EPS = 1e-16      # utils/const.py:5 (clamp of (E, pT) in polar coordinates, utils/train.py:58-65)
@@ -113,9 +113,15 @@ class GNNAETrainer:
     >>> loss = tr.step(x_host_pinned)          # float; H2D copy, graph replay, all-reduce, Adam, D2H of the loss
 
     Covers every latent map of the reference ('mean', 'max', 'min', the GLOBAL_MIX and LOCAL_MIX spellings), the decoder's
-    ``normalize_output`` (tanh), the polar-coordinate clamp of utils/train.py:55-65 (``polar_coord``) and the Chamfer and MSE
-    branches of ``get_loss`` (utils/train.py:338-361, ``loss_choice``).  Dropout and batch-norm are not part of the fused step
+    ``normalize_output`` (tanh), the polar-coordinate clamp of utils/train.py:55-65 (``polar_coord``) and the Chamfer, MSE and
+    EMD branches of ``get_loss`` (utils/train.py:330-385, ``loss_choice``).  Dropout and batch-norm are not part of the fused step
     (the reference's batch-norm path crashes; dropout > 0 raises in the modules).
+
+    ``loss_choice="emd"`` trains with the exact energy mover's distance (one gj_emd_loss solve of the whole batch per step, inside
+    the CUDA graph).  Its options come from ``emd_loss`` (default ``EMDLoss(polar_coord=polar_coord)``): R, beta, norm,
+    periodic_phi, polar_coord (must equal the trainer's) and reduction ("sum" over the jets, or "mean" over the global batch;
+    "none" raises).  Cartesian 3- / 4-vectors are converted as EMDLoss converts them; at most 150 particles per jet.  A jet whose
+    solver stops at its augmentation cap makes ``loss_from_stats`` (``step``, ``run_epoch``) raise.
 
     ``batched_launches`` (default on, used where every step runs the fused tensor-core kernels): the six message-passing steps
     run as a chain -- ONE launch packs all steps' bf16 edge-parameter images, ONE launch reduces all steps' parameter-gradient
@@ -127,7 +133,7 @@ class GNNAETrainer:
                  jet_features_weight: float = 1.0, chamfer_mode: str = "intended", encoder_metric: str = "euclidean",
                  decoder_metric: str = "euclidean", process_group=None, use_cuda_graph: bool = True,
                  loss_choice: str = "chamfer", polar_coord: bool = False, optimizer: str = "adam",
-                 batched_launches: bool = True):
+                 batched_launches: bool = True, emd_loss: Optional[EMDLoss] = None):
         self.enc, self.dec = encoder, decoder
         g_e, g_d = encoder.encoder, decoder.decoder
         dev = next(encoder.parameters()).device
@@ -153,9 +159,23 @@ class GNNAETrainer:
             self.loss_choice = "chamfer"
         elif lc in ("mse", "mseloss", "mse_loss"):
             self.loss_choice = "mse"
+        elif lc in ("emd", "emdloss", "emd_loss"):
+            self.loss_choice = "emd"
         else:
-            raise NotImplementedError(f"loss_choice {loss_choice!r}: the fused step covers the Chamfer and MSE branches of get_loss "
-                                      "(utils/train.py:338-361); the EMD loss is out of scope")
+            raise NotImplementedError(f"loss_choice {loss_choice!r}: the fused step covers the Chamfer, MSE and EMD branches of "
+                                      "get_loss (utils/train.py:330-385); 'hybrid' is not covered")
+        if self.loss_choice == "emd":
+            if emd_loss is None:
+                emd_loss = EMDLoss(polar_coord=polar_coord)
+            if emd_loss.reduction == "none":
+                raise ValueError("loss_choice='emd' needs a scalar loss: EMDLoss reduction 'sum' or 'mean', not 'none'")
+            if emd_loss.polar_coord != bool(polar_coord):
+                raise ValueError(f"EMDLoss(polar_coord={emd_loss.polar_coord}) does not match the trainer's polar_coord={polar_coord}")
+            if polar_coord and encoder.input_node_size != 3:
+                raise ValueError(f"polar_coord=True expects [pt, eta, phi] jets (3 features), got {encoder.input_node_size}")
+            if encoder.num_nodes > 150:
+                raise ValueError(f"the EMD loss supports at most 150 particles per jet, got {encoder.num_nodes}")
+            self.emd = emd_loss
         if self.loss_choice == "chamfer" and chamfer_mode == "reference" and jet_features_weight == 0:
             raise UnboundLocalError("jet_loss referenced before assignment (reference chamfer_loss.py:42)")
         # the Chamfer target is the input batch: both sides must be 3- or 4-vectors of one width (distance_sq.py:31-42)
@@ -230,14 +250,20 @@ class GNNAETrainer:
         self.world = 1
         if torch.distributed.is_available() and torch.distributed.is_initialized():
             self.world = torch.distributed.get_world_size(process_group)
+        if self.loss_choice == "emd":
+            # EMDLoss's reduction over the GLOBAL batch: with "mean" the all-reduced gradient equals the single-device one
+            self.emd_scale = 1.0 if self.emd.reduction == "sum" else 1.0 / (self.world * B)
+            self.emd_flags = (_lib.GJ_EMD_NORM if self.emd.norm else 0) | (_lib.GJ_EMD_PERIODIC_PHI if self.emd.periodic_phi else 0)
         self.jet_terms = torch.empty((B, 2), **f32)
-        self.stats = torch.zeros(8, **f32)     # [chamfer, jet, wc*chamfer + wj*jet, sum|p|, sum p^2]
+        # [chamfer | EMD, jet, loss term, sum|p|, sum p^2, EMD jets whose solver hit its cap]
+        self.stats = torch.zeros(8, **f32)
         self.stats_host = torch.zeros(8, dtype=torch.float32).pin_memory()
         ws = max([self.lib.gj_mp_step_bwd_workspace(s["desc"]) for s in self.enc_steps + self.dec_steps] +
                  [self.lib.gj_mp_step_fwd_workspace(s["desc"]) for s in self.enc_steps + self.dec_steps] +
                  [self.lib.gj_linear_bwd_workspace(B * N, max(self.latent_w, self.enc_out_w), max(self.h0, self.latent_w)),
                   self.lib.gj_linear_bwd_workspace(B, max(self.latent_w, N * self.enc_out_w), max(N * self.h0, self.latent_w)),
-                  self.lib.gj_param_norms_workspace(n), self.lib.gj_mse_workspace(), 16])
+                  self.lib.gj_param_norms_workspace(n), self.lib.gj_mse_workspace(), 16] +
+                 ([self.lib.gj_emd_loss_workspace(B, N)] if self.loss_choice == "emd" else []))
         self.ws_bytes = int(ws)
         self.ws = torch.empty((self.ws_bytes + 3) // 4, **f32)
         # per-step buffers in which the forward call leaves P|Q, the packed edge parameters and the pair distances for the
@@ -339,11 +365,16 @@ class GNNAETrainer:
             ops.LAUNCHES["count"] += 1
 
     def _loss(self, st):
-        """Chamfer terms (+ d loss / d recon) and parameter norms of the resident batch -> self.stats."""
+        """Loss terms (+ d loss / d recon) and parameter norms of the resident batch -> self.stats."""
         lib, B, N, D = self.lib, self.B, self.N, self.recon.shape[-1]
         if self.loss_choice == "mse":      # nn.MSELoss: mean over the elements of the GLOBAL batch
             _lib.check(lib.gj_mse_fwd_bwd(B * N * D, float(self.world * B * N * D), self.recon.data_ptr(), self.x.data_ptr(),
                                           self.stats.data_ptr(), self.dp.data_ptr(), self.ws.data_ptr(), self.ws_bytes, st), "mse")
+        elif self.loss_choice == "emd":    # the recon after tanh / clamp against the input, as EMDLoss sees them in the train loop
+            coords = _lib.GJ_EMD_COORDS_POLAR if self.emd.polar_coord else _lib.GJ_EMD_COORDS_CARTESIAN
+            _lib.check(lib.gj_emd_loss(B, N, D, coords, self.recon.data_ptr(), self.x.data_ptr(), self.emd.R, self.emd.beta,
+                                       self.emd_flags, self.emd_scale, self.stats.data_ptr(), self.stats.data_ptr() + 20,
+                                       self.dp.data_ptr(), self.ws.data_ptr(), self.ws_bytes, st), "emd loss")
         else:
             _lib.check(lib.gj_chamfer_fwd_bwd(B, N, N, D, _norm_id(self.recon, self.norm_choice), self.wc, self.wj,
                                               self.recon.data_ptr(), self.x.data_ptr(), self.jet_terms.data_ptr(),
@@ -465,7 +496,14 @@ class GNNAETrainer:
         self.apply_gradients()
 
     def loss_from_stats(self, stats) -> float:
-        """train.py:376-384: batch loss = chamfer value + l1_lambda * sum|p| + l2_lambda * sum p^2 (this rank's shard)."""
+        """train.py:376-384: batch loss = loss value + l1_lambda * sum|p| + l2_lambda * sum p^2 (this rank's shard).
+
+        Raises ``RuntimeError`` if the EMD solver stopped at its augmentation cap for a jet of the batch (``stats[5] > 0``): that
+        jet's EMD and gradient are not optimal.  The row is read after the step, so the parameter update of that step has already
+        been applied.  The cap leaves a margin of about 8x over the augmentation counts seen in practice (DESIGN.md section 8)."""
+        if float(stats[5]) > 0:
+            raise RuntimeError(f"EMD loss: the transport solver did not converge for {int(float(stats[5]))} jet(s) of the batch "
+                               "(the update of this step has already been applied)")
         v = float(stats[2])
         if self.l1 > 0:
             v += self.l1 * float(stats[3])

@@ -21,6 +21,7 @@
  *   gj_latent_extreme_fwd/bwd        : models/encoder.py:150-155 ('max' / 'min' latent maps)
  *   gj_output_transform_fwd/bwd      : models/decoder.py:123-124 (tanh) and utils/train.py:55-65 (polar clamp)
  *   gj_mse_fwd_bwd                   : utils/train.py:359-361 (nn.MSELoss branch of get_loss)
+ *   gj_emd_loss                      : the emd branch of get_loss (utils/train.py:330-385) on utils/losses/emd_loss.py
  *
  * Tensor layouts: all tensors are dense row-major float32 in HBM.
  *   node features  h      (B, N, H)
@@ -204,6 +205,28 @@ size_t gj_emd_workspace(int32_t batch, int32_t np_, int32_t nq);
 int gj_emd(int32_t batch, int32_t np_, int32_t nq, const float* p, const float* q, float R, float beta, int32_t flags,
            double* emd_out, double* flow_out, float* dp_out, double* potentials_out, int32_t* status_out,
            void* workspace, size_t workspace_bytes, void* stream);
+
+/* The EMD as a training loss (the `emd` branch of get_loss, utils/train.py:330-385, on utils/losses/emd_loss.py): gj_emd's solver,
+ * one CTA per jet, on the training step's layout, with the gradient scaled and in the input's own coordinates.
+ * p (B,N,D) is the reconstruction, q (B,N,D) the target, fp32, D in {3,4}:
+ *   GJ_EMD_COORDS_POLAR     : D == 3, [pt, eta, phi], as gj_emd takes them;
+ *   GJ_EMD_COORDS_CARTESIAN : (px, py, pz) or (E, px, py, pz), converted on load as losses._to_polar does
+ *                             (pt = sqrt(px^2 + py^2 + 1e-16), eta = asinh(pz / (pt + 1e-16)), phi = atan2(py + 1e-16, px + 1e-16));
+ *                             E does not enter the EMD.
+ * R, beta, flags (GJ_EMD_NORM, GJ_EMD_PERIODIC_PHI) as for gj_emd; 1 <= N <= 150.
+ * terms (3) fp32, overwritten: terms[0] = sum_b EMD_b, terms[1] = 0, terms[2] = scale * terms[0] (the slots of gj_chamfer_fwd_bwd);
+ *   the per-jet EMDs are fp64 in the workspace and summed in a fixed order (bitwise reproducible).
+ * failed (1) fp32, overwritten: number of jets whose solver stopped at the augmentation cap (their EMD and gradient are not optimal).
+ * dp (B,N,D) fp32, may be NULL: scale * dEMD_b/dp as gj_emd's dp_out (rounded to fp32 first), through the Jacobian of the
+ *   conversion in Cartesian coordinates; the E component is 0.
+ * Two launches (the solver, then the sum), no host synchronisation, capturable in a CUDA graph.  Every argument is checked on the
+ * host before any launch; workspace_bytes >= gj_emd_loss_workspace(B, N). */
+#define GJ_EMD_COORDS_POLAR 0
+#define GJ_EMD_COORDS_CARTESIAN 1
+size_t gj_emd_loss_workspace(int32_t batch, int32_t n);
+int gj_emd_loss(int32_t batch, int32_t n, int32_t dim, int32_t coords, const float* p, const float* q, float R, float beta,
+                int32_t flags, float scale, float* terms, float* failed, float* dp, void* workspace, size_t workspace_bytes,
+                void* stream);
 
 /* Flat fused Adam (torch.optim.Adam defaults: no weight decay, no amsgrad) over n floats.
  * grad_scale multiplies the incoming gradient, l1_lambda*sign(p) and 2*l2_lambda*p are added to it
