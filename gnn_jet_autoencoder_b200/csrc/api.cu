@@ -15,11 +15,8 @@ void gj_set_error(const char* fmt, ...) {
   va_end(ap);
 }
 
-static bool node_post_tc_enabled() { static const bool v = !(getenv("GJ_NODE_POST_SIMT") && atoi(getenv("GJ_NODE_POST_SIMT")) != 0); return v && !(getenv("GJ_NODE_SIMT") && atoi(getenv("GJ_NODE_SIMT")) != 0); }
-static bool node_tc_disabled() { static const bool v = getenv("GJ_NODE_SIMT") && atoi(getenv("GJ_NODE_SIMT")) != 0; return v; }
 // programmatic dependent launch of the step's kernel chain (gj_common.cuh): GJ_PDL forces a mode, unset = the default policy
 int gj_pdl_mode() { static const int v = getenv("GJ_PDL") ? atoi(getenv("GJ_PDL")) : -1; return v; }
-bool gj_tc_v1_forced() { static const bool v = getenv("GJ_TC_V1") && atoi(getenv("GJ_TC_V1")) != 0; return v; }
 
 // bitwise-reproducible parameter gradients in the bf16 mode (gj_set_deterministic): read by the backward edge launchers
 static int g_deterministic = 0;
@@ -70,7 +67,6 @@ int gj_node_post_bwd_tc_nparts(const MPLayout&);
 int gj_reduce_steps_partials(int, const MPLayout*, const float* const*, const int*, const float* const*, const int*, const float* const*,
                              const int*, float* const*, cudaStream_t);
 size_t gj_wimage_floats();
-bool gj_tc_v1_forced();
 void gj_fwd2_plan(const MPLayout&, int*, int*);
 void gj_bwd2_plan(const MPLayout&, int*, int*);
 bool gj_bwd2_supported(const MPLayout&);
@@ -154,43 +150,38 @@ struct StepWs {   // offsets in floats
 
 static bool use_tc(const MPLayout& L, int precision) { return precision == GJ_PREC_BF16 && L.Le > 1; }
 // the step runs the second-generation fused kernels (forward and backward are covered by the same widths)
-static bool edge_mat_forced() { static const int f = getenv("GJ_EDGE_MAT") ? atoi(getenv("GJ_EDGE_MAT")) : 0; return f != 0; }
 static bool tc2_path(const MPLayout& L, int precision) {
-  return !edge_mat_forced() && use_tc(L, precision) && gj_fwd2_supported(L) && gj_bwd2_supported(L) && !gj_tc_v1_forced();
+  return use_tc(L, precision) && gj_fwd2_supported(L) && gj_bwd2_supported(L);
 }
 
 static bool edge_mat(const MPLayout& L, int precision);
 // the step runs the third-generation fused kernels (two-layer edge networks [H, H], H = 64 / 128: BASELINE config 5)
 static bool tc3_path(const MPLayout& L, int precision) {
-  return !edge_mat_forced() && use_tc(L, precision) && !tc2_path(L, precision) && gj_edge3_supported(L) && !gj_tc_v1_forced();
+  return use_tc(L, precision) && !tc2_path(L, precision) && gj_edge3_supported(L);
 }
 
 // Node-level work (P|Q projections, node MLP and their adjoints) as generic GEMMs (dense.cu): wherever a node-level weight
 // matrix does not fit the fused node kernels' shared-memory plans, and for wide layers (BASELINE config 5: H >= 64), where the
 // GEMM formulation -- tcgen05 in the bf16 mode -- is the faster one
 static bool dense_node(const MPLayout& L, int precision) {
-  static const int force = getenv("GJ_DENSE_NODE") ? atoi(getenv("GJ_DENSE_NODE")) : -1;
   if (edge_mat(L, precision)) return true;
   if (tc2_path(L, precision)) return false;
   if (!gj_node_generic_fits(L)) return true;
-  if (force >= 0) return force != 0;
   int wmax = L.H > L.E[0] ? L.H : L.E[0];
   for (int m = 0; m < L.Ln; ++m) if (L.O[m] > wmax) wmax = L.O[m];
   return wmax >= 64;
 }
 
 // The edge MLP as generic GEMMs over the materialised edge rows of a chunk of jets (dense.cu): for the widths no fused edge
-// kernel has a plan for (e.g. edge_sizes [[256, 256]]); GJ_EDGE_MAT=1 forces it (tests)
+// kernel has a plan for (e.g. edge_sizes [[256, 256]])
 static bool edge_mat(const MPLayout& L, int precision) {
-  if (edge_mat_forced()) return true;
   if (tc2_path(L, precision) || tc3_path(L, precision)) return false;
   return use_tc(L, precision) ? !gj_edge_tc_fits(L) : !gj_edge_simt_fits(L, nullptr);
 }
 
 // backward of the bf16 step with both node-level adjoints on tcgen05: their partials and the edge kernel's are reduced together
 static bool node_tail_fused(const MPLayout& L, int precision) {
-  return tc2_path(L, precision) && gj_node_post_bwd_tc_supported(L) && gj_node_pre_bwd_tc_supported(L) && node_post_tc_enabled() &&
-         !node_tc_disabled();
+  return tc2_path(L, precision) && gj_node_post_bwd_tc_supported(L) && gj_node_pre_bwd_tc_supported(L);
 }
 
 // caller-owned buffer of a step whose parameter-gradient reduction is deferred (gj_mp_step_bwd_deferred): per-CTA partials of the
@@ -273,7 +264,7 @@ static int mp_step_fwd_impl(const gj_mp_desc* d, const float* h, const float* pa
   if (workspace_bytes < w.total * sizeof(float)) { gj_set_error("%s: workspace too small", who); return GJ_ERR_WORKSPACE; }
   float* ws = (float*)workspace;
   const bool emat = edge_mat(L, d->precision);
-  const bool tc2 = tc2_path(L, d->precision) && !emat;
+  const bool tc2 = tc2_path(L, d->precision);
   const bool tc3 = tc3_path(L, d->precision);
   if (saved && !tc2 && !tc3) { gj_set_error("%s: this step has nothing to save (gj_mp_step_saved_bytes is 0)", who); return GJ_ERR_INVALID; }
   if (prepacked && !(tc2 && saved)) { gj_set_error("%s: this step has no packed parameter image (gj_mp_step_partials_bytes is 0)", who); return GJ_ERR_INVALID; }
@@ -350,13 +341,13 @@ static int mp_step_bwd_impl(const gj_mp_desc* d, const float* h, const float* e,
   if (workspace_bytes < w.total * sizeof(float)) { gj_set_error("%s: workspace too small", who); return GJ_ERR_WORKSPACE; }
   float* ws = (float*)workspace;
   const bool emat = edge_mat(L, d->precision);
-  const bool tc2 = tc2_path(L, d->precision) && !emat;
+  const bool tc2 = tc2_path(L, d->precision);
   const bool tc3 = tc3_path(L, d->precision);
   if (saved && !tc2 && !tc3) { gj_set_error("%s: this step has nothing saved (gj_mp_step_saved_bytes is 0)", who); return GJ_ERR_INVALID; }
   float* pre = saved ? (float*)saved : ws;      // read-only when it is the caller's saved buffer
-  if (partials && !(node_tail_fused(L, d->precision) && !emat && saved)) {
+  if (partials && !(node_tail_fused(L, d->precision) && saved)) {
     gj_set_error("%s: this step cannot defer its reduction (gj_mp_step_partials_bytes is 0)", who); return GJ_ERR_INVALID; }
-  if (node_tail_fused(L, d->precision) && !emat) {
+  if (node_tail_fused(L, d->precision)) {
     // node MLP adjoint (also clears dP|dQ), P|Q unless saved, edge adjoint, projections' adjoint, one reduction of all partials
     int np_post = 0, np_pre = 0, np_edge = 0;
     const float* part_edge = nullptr;
@@ -386,7 +377,7 @@ static int mp_step_bwd_impl(const gj_mp_desc* d, const float* h, const float* e,
     return gj_dense_pre_bwd(L, h, params, ws + w.dpq, dh, dparams, ws + w.dense, d->precision, st);
   }
   // node MLP adjoint: de, node-path dh, node parameter gradients
-  if (tc2 && gj_node_post_bwd_tc_supported(L) && node_post_tc_enabled()) {      // bf16 mode: the node MLP adjoint on tcgen05
+  if (tc2 && gj_node_post_bwd_tc_supported(L)) {      // bf16 mode: the node MLP adjoint on tcgen05
     int nparts = 0;
     if ((rc = gj_node_post_bwd_tc(L, e, h, params, dh_out, ws + w.de, dh, ws + w.part, &nparts, nullptr, st))) return rc;
     if ((rc = gj_reduce_partials(ws + w.part, nparts, L.nparams - L.pV[0], dparams + L.pV[0], st))) return rc;
@@ -401,7 +392,7 @@ static int mp_step_bwd_impl(const gj_mp_desc* d, const float* h, const float* e,
                                  : gj_edge_bwd_simt(L, h, ws + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, st);
   if (rc) return rc;
   // first-layer projections' adjoint: dh += Wa^T dP + Wb^T dQ, dWa, dWb, db0
-  if (tc2 && gj_node_pre_bwd_tc_supported(L) && !node_tc_disabled()) {      // bf16 mode: the projections' adjoint on tcgen05
+  if (tc2 && gj_node_pre_bwd_tc_supported(L)) {      // bf16 mode: the projections' adjoint on tcgen05
     int nparts = 0;
     if ((rc = gj_node_pre_bwd_tc(L, h, params, ws + w.dpq, dh, ws + w.part, &nparts, st))) return rc;
     return gj_reduce_pre_partials(L, ws + w.part, nparts, dparams, st);
@@ -423,7 +414,7 @@ int gj_mp_step_bwd_saved(const gj_mp_desc* d, const float* h, const float* e, co
 // ---- a chain of steps: ONE launch packs every step's parameter image, ONE launch reduces every step's gradient partials ----
 size_t gj_mp_step_partials_bytes(const gj_mp_desc* d) {
   MPLayout L; const char* why;
-  if (gj_fill_arch(d, &L, &why) || L.B == 0 || !node_tail_fused(L, d->precision) || edge_mat(L, d->precision)) return 0;
+  if (gj_fill_arch(d, &L, &why) || L.B == 0 || !node_tail_fused(L, d->precision)) return 0;
   return plan_partials(L).total * sizeof(float);
 }
 

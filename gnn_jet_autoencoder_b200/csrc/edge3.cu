@@ -359,7 +359,7 @@ struct E3Slot {
   const float* st;      // staged [P_i part | de_i part] of the tile
 };
 
-template <int E0, int E1, int NWG, int S, int IC, bool PIPE>
+template <int E0, int E1, int NWG, int S, int IC>
 __global__ void __launch_bounds__(NWG * S * 128, 1) edge_bwd3_kernel(const E3Args A, const __grid_constant__ CUtensorMap tm_w) {
   using SM = Bwd3Smem<E0, E1, NWG, S, IC>;
   constexpr int C0 = SM::C0, C1 = SM::C1;
@@ -662,15 +662,10 @@ __global__ void __launch_bounds__(NWG * S * 128, 1) edge_bwd3_kernel(const E3Arg
 #pragma unroll 1
   for (int t = 0; t < ntile; ++t) {
     E1f(sA, ts);
-    if (PIPE) {
-      if (t + 1 < ntile) L0(sB, ts ^ 1);
-      E0f(sA, ts, t + 1 == ntile);
-      const E3Slot tmp = sA; sA = sB; sB = tmp;
-      ts ^= 1;
-    } else {
-      E0f(sA, ts, t + 1 == ntile);
-      if (t + 1 < ntile) L0(sA, ts);
-    }
+    if (t + 1 < ntile) L0(sB, ts ^ 1);
+    E0f(sA, ts, t + 1 == ntile);
+    const E3Slot tmp = sA; sA = sB; sB = tmp;
+    ts ^= 1;
   }
   // all of this group's MMAs have completed: the slot a record last used is kept in the record
   if (sA.pendW) { mbar_wait(bars + 2 + sA.slot, (ph_bits >> (2 + sA.slot)) & 1u); ph_bits ^= 4u << sA.slot; }
@@ -752,8 +747,7 @@ static int e3_shape(const MPLayout& L) {
   return -1;
 }
 bool gj_edge3_supported(const MPLayout& L) {
-  static const bool off = getenv("GJ_NO_EDGE3") && atoi(getenv("GJ_NO_EDGE3")) != 0;
-  return !off && e3_shape(L) >= 0 && gj_pair_dist_bwd_fits(L);
+  return e3_shape(L) >= 0 && gj_pair_dist_bwd_fits(L);
 }
 size_t gj_edge3_wimage_floats(const MPLayout& L) { return ((size_t)(e3_shape(L) == 0 ? WImage3<64, 64>::bytes : WImage3<128, 128>::bytes) + 255) / 256 * 64; }
 // forward workspace: per-j-block partial aggregates (N > 32)
@@ -824,8 +818,7 @@ template <int E0, int E1, int NWG, int S, int IC>
 static int e3_launch_bwd(E3Args& A, int grid, cudaStream_t stream) {
   using SM = Bwd3Smem<E0, E1, NWG, S, IC>;
   static_assert(SM::total <= 227 * 1024, "backward shared-memory plan");
-  static const int pipe_env = getenv("GJ_E3_PIPE") ? atoi(getenv("GJ_E3_PIPE")) : 1;
-  auto kern = pipe_env ? edge_bwd3_kernel<E0, E1, NWG, S, IC, true> : edge_bwd3_kernel<E0, E1, NWG, S, IC, false>;
+  auto kern = edge_bwd3_kernel<E0, E1, NWG, S, IC>;
   cudaError_t ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SM::total);
   if (ce != cudaSuccess) { gj_set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(ce)); return GJ_ERR_CUDA; }
   long long ng = (long long)grid * NWG;      // every (jet, j block) is shared by at most two groups (two-addend atomic dQ sums)

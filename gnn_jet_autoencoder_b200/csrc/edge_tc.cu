@@ -1119,13 +1119,11 @@ int gj_edge_fwd_tc(MPLayout L, const float* h, const float* pq, const float* par
     gj_set_error("gj_mp_step_fwd(bf16): needs %d B shared memory / %d TMEM columns (limits 232448 / 512)", T.smem_bytes, T.tmem_cols_total);
     return GJ_ERR_SMEM;
   }
-  static const int nh_env = getenv("GJ_TC_NH") ? atoi(getenv("GJ_TC_NH")) : 2;
   static const int trace_fwd = getenv("GJ_TRACE") ? atoi(getenv("GJ_TRACE")) : 0;
   T.trace = trace_fwd == 2;
   if (T.trace) { int z[4] = {0, 0, 0, 0}; cudaMemcpyToSymbolAsync(g_trace_n, z, sizeof(z), 0, cudaMemcpyHostToDevice, stream); }
-  const int NH = nh_env == 1 ? 1 : 2;
-  auto kern = NWG == 1 ? (NH == 1 ? edge_fwd_tc_kernel<1, 1> : edge_fwd_tc_kernel<1, 2>)
-                       : (NH == 1 ? edge_fwd_tc_kernel<2, 1> : edge_fwd_tc_kernel<2, 2>);
+  constexpr int NH = 2;
+  auto kern = NWG == 1 ? edge_fwd_tc_kernel<1, NH> : edge_fwd_tc_kernel<2, NH>;
   cudaError_t ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, T.smem_bytes);
   if (ce != cudaSuccess) { gj_set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(ce)); return GJ_ERR_CUDA; }
   int sms = gj_num_sms();
@@ -1170,11 +1168,10 @@ template <int E0P>
 static int launch_tc_bwd(const MPLayout& L, const BwdPlan& T, const float* h, const float* pq, const float* params,
                          const float* de, float* dpq, float* dh, float* part, int grid, cudaStream_t stream) {
   constexpr int NWG = 2;
-  // NH = 2 (256 threads per tile) is measured slower for the backward kernel: 17 warps cap the kernel at 96 registers and
-  // the first-layer adjoint spills; it stays selectable for experiments
-  static const int nh_env = getenv("GJ_TC_NH_BWD") ? atoi(getenv("GJ_TC_NH_BWD")) : 1;
-  const int NH = nh_env == 2 ? 2 : 1;
-  auto kern = NH == 1 ? edge_bwd_tc_kernel<NWG, 1, E0P> : edge_bwd_tc_kernel<NWG, 2, E0P>;
+  // NH = 1: with NH = 2 (256 threads per tile) the backward kernel is measured slower, since 17 warps cap it at 96 registers
+  // and the first-layer adjoint spills
+  constexpr int NH = 1;
+  auto kern = edge_bwd_tc_kernel<NWG, NH, E0P>;
   cudaError_t ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, T.smem_bytes);
   if (ce != cudaSuccess) { gj_set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(ce)); return GJ_ERR_CUDA; }
   kern<<<grid, NWG * 128 * NH + 32, T.smem_bytes, stream>>>(L, T, h, pq, params, de, dpq, dh, part);

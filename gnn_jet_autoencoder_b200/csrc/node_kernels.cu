@@ -387,7 +387,7 @@ __global__ void __launch_bounds__(NK_THREADS) node_post_bwd_kernel(const PostArg
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// thread-per-row forward kernels for the usual small widths (compile-time sizes: every loop unrolls, activations live in
+// thread-per-row kernels for the usual small widths (compile-time sizes: every loop unrolls, activations live in
 // registers, weights are read as warp-broadcast 16-byte shared-memory loads -> FFMA bound)
 // ---------------------------------------------------------------------------------------------------------
 #define NF_THREADS 128
@@ -430,130 +430,15 @@ __device__ __forceinline__ float4 nf_dot4_nobias(const float (&x)[KP], const flo
   return make_float4(acc[0], acc[1], acc[2], acc[3]);
 }
 
-// PQ[row][0..32) = Wa h + b0 ; PQ[row][32..64) = Wb h      (E0 = 32; KP = columns of h present in memory, padded to 4)
-template <int KP>
-__global__ void __launch_bounds__(NF_THREADS) node_pre_fwd_fast_kernel(int rows, int H, int cols, int ld, int K0, const float* __restrict__ h,
-                                                                       const float* __restrict__ w0, const float* __restrict__ b0,
-                                                                       float* __restrict__ pq) {
-  gj_pdl_sync();
-  constexpr int XS = KP + 4, OS = 36;
-  __shared__ __align__(16) float W[64 * KP];
-  __shared__ float bias[64];
-  __shared__ __align__(16) float sX[NF_THREADS * XS];
-  __shared__ __align__(16) float sO[NF_THREADS * OS];
-  for (int idx = threadIdx.x; idx < 64 * KP; idx += NF_THREADS) {
-    const int o = idx / KP, k = idx - o * KP;
-    if (k < cols) nf_cp_async4(W + idx, w0 + (o & 31) * K0 + (o < 32 ? k : H + k));
-    else W[idx] = 0.f;
-  }
-  if (threadIdx.x < 64) bias[threadIdx.x] = threadIdx.x < 32 ? __ldg(b0 + threadIdx.x) : 0.f;
-  for (int row0 = blockIdx.x * NF_THREADS; row0 < rows; row0 += gridDim.x * NF_THREADS) {
-    const int nrows = min(NF_THREADS, rows - row0);
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < nrows * KP; idx += NF_THREADS) {
-      const int r = idx / KP, k = idx - r * KP;
-      if (k < cols) nf_cp_async4(sX + r * XS + k, h + (size_t)(row0 + r) * ld + k);
-      else sX[r * XS + k] = 0.f;
-    }
-    nf_cp_async_wait();
-    __syncthreads();
-    float x[KP];
-#pragma unroll
-    for (int k = 0; k < KP; k += 4) {
-      const float4 v = *reinterpret_cast<const float4*>(sX + threadIdx.x * XS + k);
-      x[k] = v.x; x[k + 1] = v.y; x[k + 2] = v.z; x[k + 3] = v.w;
-    }
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {      // P then Q: 32 outputs per pass through the output tile
-#pragma unroll
-      for (int o0 = 0; o0 < 32; o0 += 4)
-        *reinterpret_cast<float4*>(sO + threadIdx.x * OS + o0) = nf_dot4<KP>(x, W, bias, 32 * half + o0);
-      __syncthreads();
-      for (int idx = threadIdx.x; idx < nrows * 8; idx += NF_THREADS) {
-        const int r = idx >> 3, q = idx & 7;
-        *reinterpret_cast<float4*>(pq + (size_t)(row0 + r) * 64 + 32 * half + 4 * q) = *reinterpret_cast<const float4*>(sO + r * OS + 4 * q);
-      }
-      __syncthreads();
-    }
-  }
-}
-
-// h' = leaky(V1 leaky(V0 [e | h] + c0) + c1)      (two node layers; I0P, O0P, O1P = widths padded to 4; EL = 16)
-template <int I0P, int O0P, int O1P>
-__global__ void __launch_bounds__(NF_THREADS) node_post_fwd_fast_kernel(int rows, int EL, int cols, int ld, int I0, int O0, int O1, float alpha,
-                                                                        const float* __restrict__ e, const float* __restrict__ h,
-                                                                        const float* __restrict__ V0, const float* __restrict__ c0,
-                                                                        const float* __restrict__ V1, const float* __restrict__ c1,
-                                                                        float* __restrict__ h_out) {
-  gj_pdl_sync();
-  constexpr int XS = 4 * ((I0P / 4) | 1), OS = 4 * ((O1P / 4) | 1);
-  __shared__ __align__(16) float sV0[O0P * I0P];
-  __shared__ __align__(16) float sV1[O1P * O0P];
-  __shared__ float sc0[O0P], sc1[O1P];
-  __shared__ __align__(16) float sX[NF_THREADS * XS];
-  __shared__ __align__(16) float sO[NF_THREADS * OS];
-  for (int idx = threadIdx.x; idx < O0P * I0P; idx += NF_THREADS) {
-    const int o = idx / I0P, k = idx - o * I0P;
-    if (o < O0 && k < I0) nf_cp_async4(sV0 + idx, V0 + o * I0 + k);
-    else sV0[idx] = 0.f;
-  }
-  for (int idx = threadIdx.x; idx < O1P * O0P; idx += NF_THREADS) {
-    const int o = idx / O0P, k = idx - o * O0P;
-    if (o < O1 && k < O0) nf_cp_async4(sV1 + idx, V1 + o * O0 + k);
-    else sV1[idx] = 0.f;
-  }
-  for (int o = threadIdx.x; o < O0P; o += NF_THREADS) sc0[o] = o < O0 ? __ldg(c0 + o) : 0.f;
-  for (int o = threadIdx.x; o < O1P; o += NF_THREADS) sc1[o] = o < O1 ? __ldg(c1 + o) : 0.f;
-  for (int row0 = blockIdx.x * NF_THREADS; row0 < rows; row0 += gridDim.x * NF_THREADS) {
-    const int nrows = min(NF_THREADS, rows - row0);
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < nrows * 16; idx += NF_THREADS) {      // e: 16 columns, rows contiguous
-      const int r = idx >> 4, k = idx & 15;
-      nf_cp_async4(sX + r * XS + k, e + (size_t)(row0 + r) * EL + k);
-    }
-    for (int idx = threadIdx.x; idx < nrows * (I0P - 16); idx += NF_THREADS) {
-      const int r = idx / (I0P - 16), k = idx - r * (I0P - 16);
-      if (k < cols) nf_cp_async4(sX + r * XS + 16 + k, h + (size_t)(row0 + r) * ld + k);
-      else sX[r * XS + 16 + k] = 0.f;
-    }
-    nf_cp_async_wait();
-    __syncthreads();
-    float x[I0P];
-#pragma unroll
-    for (int k = 0; k < I0P; k += 4) {
-      const float4 v = *reinterpret_cast<const float4*>(sX + threadIdx.x * XS + k);
-      x[k] = v.x; x[k + 1] = v.y; x[k + 2] = v.z; x[k + 3] = v.w;
-    }
-    float y0[O0P];
-#pragma unroll
-    for (int o0 = 0; o0 < O0P; o0 += 4) {
-      const float4 v = nf_dot4<I0P>(x, sV0, sc0, o0);
-      y0[o0] = fmaxf(v.x, alpha * v.x); y0[o0 + 1] = fmaxf(v.y, alpha * v.y); y0[o0 + 2] = fmaxf(v.z, alpha * v.z); y0[o0 + 3] = fmaxf(v.w, alpha * v.w);
-    }
-#pragma unroll
-    for (int o0 = 0; o0 < O1P; o0 += 4) {
-      const float4 v = nf_dot4<O0P>(y0, sV1, sc1, o0);
-      *reinterpret_cast<float4*>(sO + threadIdx.x * OS + o0) =
-          make_float4(fmaxf(v.x, alpha * v.x), fmaxf(v.y, alpha * v.y), fmaxf(v.z, alpha * v.z), fmaxf(v.w, alpha * v.w));
-    }
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < nrows * O1; idx += NF_THREADS) {
-      const int r = idx / O1, o = idx - r * O1;
-      h_out[(size_t)(row0 + r) * O1 + o] = sO[r * OS + o];
-    }
-  }
-}
-
 // ---------------------------------------------------------------------------------------------------------
-// Warp-autonomous versions of the two forward kernels above (the ones the steps launch; GJ_NODE_FWD_V1=1 selects the CTA-tile
-// kernels).  The CTA-tile kernels run one serial chain per 128-row tile -- stage weights, stage the tile, compute, store, with
-// CTA-wide barriers in between -- on 592-960 CTAs, each of which re-stages the weights: 3-6x their HBM / FFMA floor.  Here a CTA
-// of 8 warps stages the weights ONCE and every warp then walks its own 32-row tiles with no CTA-wide synchronisation: the next
-// tile's rows are fetched (cp.async, 16-byte pieces where the layout allows) into the warp's staging rows as soon as every lane
-// holds its row in registers, so the fetch runs under the ~2000 FFMA / LDS of the current tile; outputs leave as 16-byte
-// coalesced stores (a tile's output rows are one contiguous block).  Tiles are dealt round-robin to CTAs first, then to the
-// warps of a CTA, so every SM gets the same number of tiles (+-1).  Per-row arithmetic is the code of the kernels above
-// (nf_dot4 in the same order): results are bitwise identical.
+// Warp-autonomous forward kernels (projections and node MLP).  A CTA-wide tile loop would run one serial chain per 128-row
+// tile -- stage weights, stage the tile, compute, store, with CTA-wide barriers in between -- on 592-960 CTAs, each of which
+// re-stages the weights: 3-6x the HBM / FFMA floor.  Here a CTA of 8 warps stages the weights ONCE and every warp then walks
+// its own 32-row tiles with no CTA-wide synchronisation: the next tile's rows are fetched (cp.async, 16-byte pieces where the
+// layout allows) into the warp's staging rows as soon as every lane holds its row in registers, so the fetch runs under the
+// ~2000 FFMA / LDS of the current tile; outputs leave as 16-byte coalesced stores (a tile's output rows are one contiguous
+// block).  Tiles are dealt round-robin to CTAs first, then to the warps of a CTA, so every SM gets the same number of tiles
+// (+-1).
 // ---------------------------------------------------------------------------------------------------------
 #define NW_WARPS 8
 __device__ __forceinline__ void nf_cp_async16(float* dst, const float* src) {
@@ -605,7 +490,7 @@ struct NwPreSmem {
   static constexpr int bytes = (o_warp + NW_WARPS * warp_floats) * 4;
 };
 
-// PQ[row][0..32) = Wa h + b0 ; PQ[row][32..64) = Wb h      (node_pre_fwd_fast_kernel, warp-autonomous)
+// PQ[row][0..32) = Wa h + b0 ; PQ[row][32..64) = Wb h      (E0 = 32; KP = columns of h present in memory, padded to 4)
 template <int KP>
 __global__ void __launch_bounds__(NW_WARPS * 32, 2) node_pre_fwd_warp_kernel(int rows, int H, int cols, int ld, int K0,
                                                                             const float* __restrict__ h, const float* __restrict__ w0,
@@ -672,7 +557,7 @@ struct NwPostSmem {
   static constexpr int bytes = (o_warp + NW_WARPS * warp_floats) * 4;
 };
 
-// h' = leaky(V1 leaky(V0 [e | h] + c0) + c1)      (node_post_fwd_fast_kernel, warp-autonomous)
+// h' = leaky(V1 leaky(V0 [e | h] + c0) + c1)      (two node layers; I0P, O0P, O1P = widths padded to 4; EL = 16)
 template <int I0P, int O0P, int O1P>
 __global__ void __launch_bounds__(NW_WARPS * 32, 2) node_post_fwd_warp_kernel(int rows, int EL, int cols, int ld, int I0, int O0, int O1,
                                                                              float alpha, const float* __restrict__ e,
@@ -1124,13 +1009,7 @@ static int nk_set_smem(K kern, int bytes) {
   return GJ_OK;
 }
 
-static int nf_grid(int rows) {
-  int blocks = (rows + NF_THREADS - 1) / NF_THREADS, cap = gj_num_sms() * 4;
-  return blocks < cap ? (blocks > 0 ? blocks : 1) : cap;
-}
-
 // warp-autonomous forward kernels: CTAs of NW_WARPS warps, two per SM, tiles of 32 rows dealt round-robin
-static bool nw_disabled() { static const bool v = getenv("GJ_NODE_FWD_V1") && atoi(getenv("GJ_NODE_FWD_V1")) != 0; return v; }
 static int nw_grid(int rows) {
   const int tiles = (rows + 31) / 32, cap = gj_num_sms() * 2;
   const int blocks = (tiles + NW_WARPS - 1) / NW_WARPS;
@@ -1158,22 +1037,13 @@ static int nw_post_launch(const MPLayout& L, const float* e, const float* h, con
 
 int gj_node_pre_fwd(const MPLayout& L, const float* h, const float* params, float* pq, cudaStream_t st) {
   if (L.E[0] == 32 && L.E0p == 32 && L.cols <= 32) {      // thread-per-row kernel (the usual first edge width)
-    const int rows = L.B * L.N, kp = L.cols <= 4 ? 4 : (L.cols <= 8 ? 8 : (L.cols <= 16 ? 16 : 32));
+    const int kp = L.cols <= 4 ? 4 : (L.cols <= 8 ? 8 : (L.cols <= 16 ? 16 : 32));
     const float* w0 = params + L.pW[0];
     const float* b0 = params + L.pb[0];
-    if (!nw_disabled()) {
-      if (kp == 4) return nw_pre_launch<4>(L, h, w0, b0, pq, st);
-      if (kp == 8) return nw_pre_launch<8>(L, h, w0, b0, pq, st);
-      if (kp == 16) return nw_pre_launch<16>(L, h, w0, b0, pq, st);
-      return nw_pre_launch<32>(L, h, w0, b0, pq, st);
-    }
-    const int grid = nf_grid(rows);
-    if (kp == 4) gj_launch(node_pre_fwd_fast_kernel<4>, grid, NF_THREADS, 0, st, rows, L.H, L.cols, L.ld, L.K[0], h, w0, b0, pq);
-    else if (kp == 8) gj_launch(node_pre_fwd_fast_kernel<8>, grid, NF_THREADS, 0, st, rows, L.H, L.cols, L.ld, L.K[0], h, w0, b0, pq);
-    else if (kp == 16) gj_launch(node_pre_fwd_fast_kernel<16>, grid, NF_THREADS, 0, st, rows, L.H, L.cols, L.ld, L.K[0], h, w0, b0, pq);
-    else gj_launch(node_pre_fwd_fast_kernel<32>, grid, NF_THREADS, 0, st, rows, L.H, L.cols, L.ld, L.K[0], h, w0, b0, pq);
-    NK_CHECK_LAUNCH("node_pre_fwd launch");
-    return GJ_OK;
+    if (kp == 4) return nw_pre_launch<4>(L, h, w0, b0, pq, st);
+    if (kp == 8) return nw_pre_launch<8>(L, h, w0, b0, pq, st);
+    if (kp == 16) return nw_pre_launch<16>(L, h, w0, b0, pq, st);
+    return nw_pre_launch<32>(L, h, w0, b0, pq, st);
   }
   PreArgs A; int bytes = pre_plan(L, &A, false);
   if (bytes < 0) { gj_set_error("node_pre_fwd: widths do not fit shared memory"); return GJ_ERR_SMEM; }
@@ -1255,29 +1125,13 @@ int gj_node_pre_bwd(const MPLayout& L, const float* h, const float* params, cons
   return GJ_OK;
 }
 
-template <int I0P, int O0P, int O1P>
-static void nf_post_launch(const MPLayout& L, const float* e, const float* h, const float* params, float* h_out, cudaStream_t st) {
-  const int rows = L.B * L.N;
-  gj_launch(node_post_fwd_fast_kernel<I0P, O0P, O1P>, nf_grid(rows), NF_THREADS, 0, st,
-      rows, L.EL, L.cols, L.ld, L.I[0], L.O[0], L.O[1], L.alpha, e, h, params + L.pV[0], params + L.pc[0], params + L.pV[1], params + L.pc[1], h_out);
-}
-
 int gj_node_post_fwd(const MPLayout& L, const float* e, const float* h, const float* params, float* h_out, cudaStream_t st) {
   if (L.Ln == 2 && L.EL == 16 && L.alpha <= 1.f && L.cols <= L.H) {      // thread-per-row kernels for the usual node widths
     const int i0p = (L.I[0] + 3) & ~3, o0p = (L.O[0] + 3) & ~3, o1p = (L.O[1] + 3) & ~3;
-    if (!nw_disabled()) {
-      if (i0p == 32 && o0p == 16 && o1p == 32) return nw_post_launch<32, 16, 32>(L, e, h, params, h_out, st);
-      if (i0p == 48 && o0p == 32 && o1p == 8) return nw_post_launch<48, 32, 8>(L, e, h, params, h_out, st);
-      if (i0p == 24 && o0p == 8 && o1p == 20) return nw_post_launch<24, 8, 20>(L, e, h, params, h_out, st);
-      if (i0p == 24 && o0p == 8 && o1p == 4) return nw_post_launch<24, 8, 4>(L, e, h, params, h_out, st);
-    }
-    bool done = true;
-    if (i0p == 32 && o0p == 16 && o1p == 32) nf_post_launch<32, 16, 32>(L, e, h, params, h_out, st);
-    else if (i0p == 48 && o0p == 32 && o1p == 8) nf_post_launch<48, 32, 8>(L, e, h, params, h_out, st);
-    else if (i0p == 24 && o0p == 8 && o1p == 20) nf_post_launch<24, 8, 20>(L, e, h, params, h_out, st);
-    else if (i0p == 24 && o0p == 8 && o1p == 4) nf_post_launch<24, 8, 4>(L, e, h, params, h_out, st);
-    else done = false;
-    if (done) { NK_CHECK_LAUNCH("node_post_fwd launch"); return GJ_OK; }
+    if (i0p == 32 && o0p == 16 && o1p == 32) return nw_post_launch<32, 16, 32>(L, e, h, params, h_out, st);
+    if (i0p == 48 && o0p == 32 && o1p == 8) return nw_post_launch<48, 32, 8>(L, e, h, params, h_out, st);
+    if (i0p == 24 && o0p == 8 && o1p == 20) return nw_post_launch<24, 8, 20>(L, e, h, params, h_out, st);
+    if (i0p == 24 && o0p == 8 && o1p == 4) return nw_post_launch<24, 8, 4>(L, e, h, params, h_out, st);
   }
   PostArgs A; int bytes = post_plan(L, &A, false);
   if (bytes < 0) { gj_set_error("node_post_fwd: widths do not fit shared memory"); return GJ_ERR_SMEM; }

@@ -595,8 +595,7 @@ void gj_set_error(const char* fmt, ...);
 
 bool gj_node_pre_bwd_tc_supported(const MPLayout& L) { return L.E[0] == 32 && L.E0p == 32 && L.cols <= 32; }
 static int pre_bwd_tc_grid(const MPLayout& L) {      // every CTA gets the same number of tiles (+-1) with 3-4 CTAs per SM resident
-  static const int env_cap = getenv("GJ_NTC_PRE_CAP") ? atoi(getenv("GJ_NTC_PRE_CAP")) : 0;      // tuning sweep (tools/gpu_ntc.sh)
-  const int tiles = (L.B * L.N + 127) / 128, cap = (env_cap > 0 ? env_cap : (L.cols <= 16 ? 4 : 3)) * gj_num_sms();
+  const int tiles = (L.B * L.N + 127) / 128, cap = (L.cols <= 16 ? 4 : 3) * gj_num_sms();
   if (tiles <= cap) return tiles > 0 ? tiles : 1;
   const int rounds = (tiles + cap - 1) / cap;
   return (tiles + rounds - 1) / rounds;
@@ -638,8 +637,7 @@ static int post_tc_shape(const MPLayout& L) {      // index of the compiled (I0P
 }
 bool gj_node_post_bwd_tc_supported(const MPLayout& L) { return post_tc_shape(L) >= 0; }
 static int post_bwd_tc_grid(const MPLayout& L) {
-  static const int env_cap = getenv("GJ_NTC_POST_CAP") ? atoi(getenv("GJ_NTC_POST_CAP")) : 0;      // tuning sweep (tools/gpu_ntc.sh)
-  const int tiles = (L.B * L.N + 127) / 128, cap = (env_cap > 0 ? env_cap : 4) * gj_num_sms();
+  const int tiles = (L.B * L.N + 127) / 128, cap = 4 * gj_num_sms();
   if (tiles <= cap) return tiles > 0 ? tiles : 1;
   const int rounds = (tiles + cap - 1) / cap;
   return (tiles + rounds - 1) / rounds;

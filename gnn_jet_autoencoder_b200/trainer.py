@@ -13,7 +13,6 @@ two Adams) as a fixed sequence of fused kernels over flat buffers.
 """
 from __future__ import annotations
 
-import os
 from collections import OrderedDict
 from typing import Optional
 
@@ -276,8 +275,6 @@ class GNNAETrainer:
         # the backward pass (each step keeps its partials in its own buffer until then) -- where every step supports it
         all_steps = self.enc_steps + self.dec_steps
         pbytes = [int(self.lib.gj_mp_step_partials_bytes(s_["desc"])) for s_ in all_steps]
-        if os.environ.get("GNNJET_BATCHED_LAUNCHES", "1") == "0":      # A/B switch (tools/)
-            batched_launches = False
         self.batched = bool(batched_launches) and all(b > 0 for b in pbytes) and all(s_["saved"] is not None for s_ in all_steps)
         for s_, nb in zip(all_steps, pbytes):
             s_["partials"] = torch.empty((nb + 3) // 4, **f32) if self.batched else None

@@ -165,9 +165,9 @@ def test_mp_step_matches_oracle(precision, N, H, edge, node, B, metric):
 
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
 def test_wide_step_matches_oracle(precision):
-    """H = 128 with a [128, 128] edge network (BASELINE config 5's middle width): the step runs on the wide-layer fall-backs
-    (half row tiles in the fp32 edge kernel, one warpgroup per CTA in the generic tensor-core forward; fp32 edge backward with
-    gradient accumulators in global memory and weights read in place; node adjoints that re-stage V / V^T per GEMM)."""
+    """H = 128 with a [128, 128] edge network (BASELINE config 5's middle width): the node level runs as generic GEMMs (dense.cu)
+    in both modes; the edge network runs on the materialised, chunked edge path of dense.cu in fp32 (the fp32 edge kernels have
+    no shared-memory plan for these widths) and on the third-generation fused kernels (edge3.cu) in bf16."""
     N, H, edge, node, B = 12, 128, [128, 128], [128, 8], 3
     rng = np.random.default_rng(128)
     shapes_e = [(o, i) for i, o in zip([2 * H + 1] + edge[:-1], edge)]

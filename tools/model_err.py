@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """bf16-mode error of the whole model against the golden fixtures (GPU box): latent / reconstruction / concatenated gradient,
-L2-relative, per golden case.  GJ_NODE_SIMT=1 shows the same numbers with the fp32 SIMT node adjoints."""
+L2-relative, per golden case."""
 import os
 import sys
 
