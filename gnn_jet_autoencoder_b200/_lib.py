@@ -15,6 +15,7 @@ GJ_PREC_FP32, GJ_PREC_BF16 = 0, 1
 GJ_METRIC_EUCLIDEAN, GJ_METRIC_MINKOWSKIAN = 0, 1
 GJ_EMD_NORM, GJ_EMD_PERIODIC_PHI = 1, 2
 GJ_EMD_COORDS_POLAR, GJ_EMD_COORDS_CARTESIAN = 0, 1
+GJ_HMSE_ABS_CARTESIAN, GJ_HMSE_ABS_POLAR, GJ_HMSE_REL_POLAR, GJ_HMSE_REL_CARTESIAN = 0, 1, 2, 3
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libgnnjet_b200.so")
@@ -63,6 +64,8 @@ SIGNATURES = {
     "gj_emd": (C.c_int, [_I, _I, _I, _P, _P, _F, _F, _I, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "gj_emd_loss_workspace": (_SZ, [_I, _I]),
     "gj_emd_loss": (C.c_int, [_I, _I, _I, _I, _P, _P, _F, _F, _I, _F, _P, _P, _P, _P, _SZ, _P]),
+    "gj_hungarian_mse_loss_workspace": (_SZ, [_I, _I]),
+    "gj_hungarian_mse_loss": (C.c_int, [_I, _I, _I, _I, _P, _P, _F, _P, _P, _P, _P, _SZ, _P]),
     "gj_adam_step_flat": (C.c_int, [_P, _P, _P, _P, _SZ, _F, _F, _F, _F, _I, _F, _F, _F, _P]),
     "gj_param_norms": (C.c_int, [_P, _SZ, _P, _P, _SZ, _P]),
     "gj_optimizer_step_flat": (C.c_int, [_I, _P, _P, _P, _P, _SZ, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _P]),

@@ -108,6 +108,9 @@ int gj_emd_launch(int, int, int, const float*, const float*, float, float, int, 
 size_t gj_emd_loss_ws_bytes(int);
 int gj_emd_loss_check(int, int, int, int, float, float, int, size_t);
 int gj_emd_loss_launch(int, int, int, int, const float*, const float*, float, float, int, float, float*, float*, float*, void*, cudaStream_t);
+size_t gj_hmse_ws_bytes(int);
+int gj_hmse_check(int, int, int, int, size_t);
+int gj_hmse_launch(int, int, int, int, const float*, const float*, float, float*, float*, int*, void*, cudaStream_t);
 int gj_linear_fwd_launch(int, int, int, const float*, const float*, const float*, float*, cudaStream_t);
 size_t gj_linear_bwd_ws_bytes(int, int, int);
 int gj_linear_bwd_launch(int, int, int, const float*, const float*, const float*, float*, float*, float*, void*, size_t, cudaStream_t);
@@ -507,6 +510,16 @@ int gj_emd_loss(int32_t batch, int32_t n, int32_t dim, int32_t coords, const flo
   if (int rc = gj_emd_loss_check(batch, n, dim, coords, R, beta, flags, workspace_bytes)) return rc;
   if (!terms || !failed || (batch > 0 && (!p || !q || !workspace))) { gj_set_error("gj_emd_loss: null pointer"); return GJ_ERR_INVALID; }
   return gj_emd_loss_launch(batch, n, dim, coords, p, q, R, beta, flags, scale, terms, failed, dp, workspace, (cudaStream_t)stream);
+}
+
+size_t gj_hungarian_mse_loss_workspace(int32_t batch, int32_t) { return gj_hmse_ws_bytes(batch); }
+
+int gj_hungarian_mse_loss(int32_t batch, int32_t n, int32_t dim, int32_t coords, const float* p, const float* q, float scale,
+                          float* terms, float* dp, int32_t* col_for_row, void* workspace, size_t workspace_bytes, void* stream) {
+  g_err[0] = 0;
+  if (int rc = gj_hmse_check(batch, n, dim, coords, workspace_bytes)) return rc;
+  if (!terms || (batch > 0 && (!p || !q || !dp || !workspace))) { gj_set_error("gj_hungarian_mse_loss: null pointer"); return GJ_ERR_INVALID; }
+  return gj_hmse_launch(batch, n, dim, coords, p, q, scale, terms, dp, col_for_row, workspace, (cudaStream_t)stream);
 }
 
 int gj_linear_fwd(int32_t rows, int32_t in_f, int32_t out_f, const float* x, const float* w, const float* b, float* y,

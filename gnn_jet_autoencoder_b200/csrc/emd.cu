@@ -303,17 +303,10 @@ __global__ void emd_kernel(int np_, int nq, float r, float beta, int norm, int p
   }
 }
 
-// losses._to_polar of one Cartesian momentum, operation by operation and without contraction, so that the solver sees the values
-// torch computes: pt = sqrt(px^2 + py^2 + eps), eta = asinh(pz / (pt + eps)), phi = atan2(py + eps, px + eps)
-__device__ __forceinline__ float3 emd_to_polar(float px, float py, float pz) {
-  const float pt = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(px, px), __fmul_rn(py, py)), GJ_EPS));
-  return make_float3(pt, asinhf(__fdiv_rn(pz, __fadd_rn(pt, GJ_EPS))), atan2f(__fadd_rn(py, GJ_EPS), __fadd_rn(px, GJ_EPS)));
-}
-
 // (pt, eta, phi) of particle k of a (.., dim) jet: the first three features (polar) or converted from the last three (Cartesian)
 __device__ __forceinline__ float3 emd_load_polar(const float* __restrict__ x, int k, int dim, int cartesian) {
   const float* e = x + (size_t)k * dim;
-  if (cartesian) return emd_to_polar(__ldg(e + dim - 3), __ldg(e + dim - 2), __ldg(e + dim - 1));
+  if (cartesian) return gj_to_polar(__ldg(e + dim - 3), __ldg(e + dim - 2), __ldg(e + dim - 1));
   return make_float3(__ldg(e), __ldg(e + 1), __ldg(e + 2));
 }
 
@@ -345,18 +338,14 @@ __global__ void emd_loss_kernel(int n, int dim, int cartesian, float r, float be
     const double g0 = (double)(float)gw * s, g1 = (double)(float)ge * s, g2 = (double)(float)gp * s;
     float* o = dp + ((size_t)b * n + tid) * dim;
     if (!cartesian) { o[0] = (float)g0; o[1] = (float)g1; o[2] = (float)g2; return; }
-    // chain rule through emd_to_polar; the energy of a 4-vector does not enter the EMD
+    // chain rule through gj_to_polar; the energy of a 4-vector does not enter the EMD
     const float* e = pg + (size_t)tid * dim + dim - 3;
-    const float px = __ldg(e), py = __ldg(e + 1), pz = __ldg(e + 2);
-    const float pt = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(px, px), __fmul_rn(py, py)), GJ_EPS));
-    const double den = (double)__fadd_rn(pt, GJ_EPS), sh = (double)__fdiv_rn(pz, __fadd_rn(pt, GJ_EPS));
-    const double deta = g1 / sqrt(1.0 + sh * sh);                       // d/d(pz / (pt + eps))
-    const double gpt = g0 - deta * sh / den;                              // total d/dpt
-    const double xe = (double)__fadd_rn(px, GJ_EPS), ye = (double)__fadd_rn(py, GJ_EPS), r2 = xe * xe + ye * ye;
+    double gx, gy, gz;
+    gj_to_polar_grad(__ldg(e), __ldg(e + 1), __ldg(e + 2), g0, g1, g2, gx, gy, gz);
     if (dim == 4) o[0] = 0.f;
-    o[dim - 3] = (float)(gpt * (double)px / (double)pt - g2 * ye / r2);
-    o[dim - 2] = (float)(gpt * (double)py / (double)pt + g2 * xe / r2);
-    o[dim - 1] = (float)(deta / den);
+    o[dim - 3] = (float)gx;
+    o[dim - 2] = (float)gy;
+    o[dim - 1] = (float)gz;
   }
 }
 

@@ -150,4 +150,24 @@ __device__ __forceinline__ float gj_warp_sum(float v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
+
+// losses._to_polar of one Cartesian momentum, operation by operation and without contraction, so that a loss kernel sees the
+// values torch computes: pt = sqrt(px^2 + py^2 + eps), eta = asinh(pz / (pt + eps)), phi = atan2(py + eps, px + eps)
+__device__ __forceinline__ float3 gj_to_polar(float px, float py, float pz) {
+  const float pt = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(px, px), __fmul_rn(py, py)), GJ_EPS));
+  return make_float3(pt, asinhf(__fdiv_rn(pz, __fadd_rn(pt, GJ_EPS))), atan2f(__fadd_rn(py, GJ_EPS), __fadd_rn(px, GJ_EPS)));
+}
+
+// Chain rule through gj_to_polar: the gradient (g_pt, g_eta, g_phi) at (px, py, pz) in fp64 -> (d/dpx, d/dpy, d/dpz)
+__device__ __forceinline__ void gj_to_polar_grad(float px, float py, float pz, double g0, double g1, double g2, double& gx,
+                                                 double& gy, double& gz) {
+  const float pt = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(px, px), __fmul_rn(py, py)), GJ_EPS));
+  const double den = (double)__fadd_rn(pt, GJ_EPS), sh = (double)__fdiv_rn(pz, __fadd_rn(pt, GJ_EPS));
+  const double deta = g1 / sqrt(1.0 + sh * sh);                       // d/d(pz / (pt + eps))
+  const double gpt = g0 - deta * sh / den;                              // total d/dpt
+  const double xe = (double)__fadd_rn(px, GJ_EPS), ye = (double)__fadd_rn(py, GJ_EPS), r2 = xe * xe + ye * ye;
+  gx = gpt * (double)px / (double)pt - g2 * ye / r2;
+  gy = gpt * (double)py / (double)pt + g2 * xe / r2;
+  gz = deta / den;
+}
 #endif

@@ -1,4 +1,4 @@
-"""The batch body of reference utils/train.py:51-85 (encoder -> decoder -> Chamfer / MSE / EMD (+L1/L2) -> backward ->
+"""The batch body of reference utils/train.py:51-85 (encoder -> decoder -> Chamfer / MSE / EMD / Hungarian MSE (+L1/L2) -> backward ->
 two Adams) as a fixed sequence of fused kernels over flat buffers.
 
 * all parameters of encoder and decoder live in ONE flat fp32 buffer (the nn.Linear parameters are
@@ -112,8 +112,8 @@ class GNNAETrainer:
     >>> loss = tr.step(x_host_pinned)          # float; H2D copy, graph replay, all-reduce, Adam, D2H of the loss
 
     Covers every latent map of the reference ('mean', 'max', 'min', the GLOBAL_MIX and LOCAL_MIX spellings), the decoder's
-    ``normalize_output`` (tanh), the polar-coordinate clamp of utils/train.py:55-65 (``polar_coord``) and the Chamfer, MSE and
-    EMD branches of ``get_loss`` (utils/train.py:330-385, ``loss_choice``).  Dropout and batch-norm are not part of the fused step
+    ``normalize_output`` (tanh), the polar-coordinate clamp of utils/train.py:55-65 (``polar_coord``) and the Chamfer, MSE,
+    EMD and Hungarian MSE branches of ``get_loss`` (utils/train.py:330-385, ``loss_choice``).  Dropout and batch-norm are not part of the fused step
     (the reference's batch-norm path crashes; dropout > 0 raises in the modules).
 
     ``loss_choice="emd"`` trains with the exact energy mover's distance (one gj_emd_loss solve of the whole batch per step, inside
@@ -121,6 +121,12 @@ class GNNAETrainer:
     periodic_phi, polar_coord (must equal the trainer's) and reduction ("sum" over the jets, or "mean" over the global batch;
     "none" raises).  Cartesian 3- / 4-vectors are converted as EMDLoss converts them; at most 150 particles per jet.  A jet whose
     solver stops at its augmentation cap makes ``loss_from_stats`` (``step``, ``run_epoch``) raise.
+
+    ``loss_choice="hungarian"`` trains with the Hungarian-matched MSE of ``HungarianMSELoss`` (one gj_hungarian_mse_loss launch of the
+    whole batch per step, inside the CUDA graph): the step computes ``HungarianMSELoss()(recon, x, abs_coord=hungarian_abs_coord,
+    polar_coord=hungarian_polar_coord)`` on the reconstruction after tanh and the polar clamp, the mean over the B N D' elements of
+    the global batch (D' = the input width in absolute Cartesian coordinates, else 3).  No gradient flows through the matching.  At
+    most 220 particles per jet.
 
     ``batched_launches`` (default on, used where every step runs the fused tensor-core kernels): the six message-passing steps
     run as a chain -- ONE launch packs all steps' bf16 edge-parameter images, ONE launch reduces all steps' parameter-gradient
@@ -132,7 +138,8 @@ class GNNAETrainer:
                  jet_features_weight: float = 1.0, chamfer_mode: str = "intended", encoder_metric: str = "euclidean",
                  decoder_metric: str = "euclidean", process_group=None, use_cuda_graph: bool = True,
                  loss_choice: str = "chamfer", polar_coord: bool = False, optimizer: str = "adam",
-                 batched_launches: bool = True, emd_loss: Optional[EMDLoss] = None):
+                 batched_launches: bool = True, emd_loss: Optional[EMDLoss] = None, hungarian_abs_coord: bool = True,
+                 hungarian_polar_coord: bool = False):
         self.enc, self.dec = encoder, decoder
         g_e, g_d = encoder.encoder, decoder.decoder
         dev = next(encoder.parameters()).device
@@ -160,9 +167,11 @@ class GNNAETrainer:
             self.loss_choice = "mse"
         elif lc in ("emd", "emdloss", "emd_loss"):
             self.loss_choice = "emd"
+        elif lc in ("hungarian", "hungarian_mse", "hungarianmse", "hungarian_mse_loss", "hungarianmseloss"):
+            self.loss_choice = "hungarian"
         else:
-            raise NotImplementedError(f"loss_choice {loss_choice!r}: the fused step covers the Chamfer, MSE and EMD branches of "
-                                      "get_loss (utils/train.py:330-385); 'hybrid' is not covered")
+            raise NotImplementedError(f"loss_choice {loss_choice!r}: the fused step covers the Chamfer, MSE, EMD and Hungarian MSE "
+                                      "branches of get_loss (utils/train.py:330-385); 'hybrid' is not covered")
         if self.loss_choice == "emd":
             if emd_loss is None:
                 emd_loss = EMDLoss(polar_coord=polar_coord)
@@ -175,6 +184,11 @@ class GNNAETrainer:
             if encoder.num_nodes > 150:
                 raise ValueError(f"the EMD loss supports at most 150 particles per jet, got {encoder.num_nodes}")
             self.emd = emd_loss
+        if self.loss_choice == "hungarian":
+            if encoder.num_nodes > 220:
+                raise ValueError(f"the Hungarian MSE loss supports at most 220 particles per jet, got {encoder.num_nodes}")
+            self.hmse_coords = ((_lib.GJ_HMSE_ABS_POLAR if hungarian_polar_coord else _lib.GJ_HMSE_ABS_CARTESIAN) if hungarian_abs_coord
+                                else (_lib.GJ_HMSE_REL_POLAR if hungarian_polar_coord else _lib.GJ_HMSE_REL_CARTESIAN))
         if self.loss_choice == "chamfer" and chamfer_mode == "reference" and jet_features_weight == 0:
             raise UnboundLocalError("jet_loss referenced before assignment (reference chamfer_loss.py:42)")
         # the Chamfer target is the input batch: both sides must be 3- or 4-vectors of one width (distance_sq.py:31-42)
@@ -253,8 +267,12 @@ class GNNAETrainer:
             # EMDLoss's reduction over the GLOBAL batch: with "mean" the all-reduced gradient equals the single-device one
             self.emd_scale = 1.0 if self.emd.reduction == "sum" else 1.0 / (self.world * B)
             self.emd_flags = (_lib.GJ_EMD_NORM if self.emd.norm else 0) | (_lib.GJ_EMD_PERIODIC_PHI if self.emd.periodic_phi else 0)
+        if self.loss_choice == "hungarian":
+            # nn.functional.mse_loss's mean over the B N D' elements of the GLOBAL batch, as the MSE branch
+            d_loss = D if self.hmse_coords == _lib.GJ_HMSE_ABS_CARTESIAN else 3
+            self.hmse_scale = 1.0 / (self.world * B * N * d_loss)
         self.jet_terms = torch.empty((B, 2), **f32)
-        # [chamfer | EMD, jet, loss term, sum|p|, sum p^2, EMD jets whose solver hit its cap]
+        # [chamfer | EMD | Hungarian squared error, jet, loss term, sum|p|, sum p^2, EMD jets whose solver hit its cap]
         self.stats = torch.zeros(8, **f32)
         self.stats_host = torch.zeros(8, dtype=torch.float32).pin_memory()
         ws = max([self.lib.gj_mp_step_bwd_workspace(s["desc"]) for s in self.enc_steps + self.dec_steps] +
@@ -262,7 +280,8 @@ class GNNAETrainer:
                  [self.lib.gj_linear_bwd_workspace(B * N, max(self.latent_w, self.enc_out_w), max(self.h0, self.latent_w)),
                   self.lib.gj_linear_bwd_workspace(B, max(self.latent_w, N * self.enc_out_w), max(N * self.h0, self.latent_w)),
                   self.lib.gj_param_norms_workspace(n), self.lib.gj_mse_workspace(), 16] +
-                 ([self.lib.gj_emd_loss_workspace(B, N)] if self.loss_choice == "emd" else []))
+                 ([self.lib.gj_emd_loss_workspace(B, N)] if self.loss_choice == "emd" else []) +
+                 ([self.lib.gj_hungarian_mse_loss_workspace(B, N)] if self.loss_choice == "hungarian" else []))
         self.ws_bytes = int(ws)
         self.ws = torch.empty((self.ws_bytes + 3) // 4, **f32)
         # per-step buffers in which the forward call leaves P|Q, the packed edge parameters and the pair distances for the
@@ -372,6 +391,10 @@ class GNNAETrainer:
             _lib.check(lib.gj_emd_loss(B, N, D, coords, self.recon.data_ptr(), self.x.data_ptr(), self.emd.R, self.emd.beta,
                                        self.emd_flags, self.emd_scale, self.stats.data_ptr(), self.stats.data_ptr() + 20,
                                        self.dp.data_ptr(), self.ws.data_ptr(), self.ws_bytes, st), "emd loss")
+        elif self.loss_choice == "hungarian":    # likewise, as HungarianMSELoss sees them
+            _lib.check(lib.gj_hungarian_mse_loss(B, N, D, self.hmse_coords, self.recon.data_ptr(), self.x.data_ptr(), self.hmse_scale,
+                                                 self.stats.data_ptr(), self.dp.data_ptr(), None, self.ws.data_ptr(), self.ws_bytes, st),
+                       "hungarian mse loss")
         else:
             _lib.check(lib.gj_chamfer_fwd_bwd(B, N, N, D, _norm_id(self.recon, self.norm_choice), self.wc, self.wj,
                                               self.recon.data_ptr(), self.x.data_ptr(), self.jet_terms.data_ptr(),

@@ -22,6 +22,7 @@
  *   gj_output_transform_fwd/bwd      : models/decoder.py:123-124 (tanh) and utils/train.py:55-65 (polar clamp)
  *   gj_mse_fwd_bwd                   : utils/train.py:359-361 (nn.MSELoss branch of get_loss)
  *   gj_emd_loss                      : the emd branch of get_loss (utils/train.py:330-385) on utils/losses/emd_loss.py
+ *   gj_hungarian_mse_loss            : utils/losses/hungarian_mse/hungarian_mse.py:27-58 as a training loss
  *
  * Tensor layouts: all tensors are dense row-major float32 in HBM.
  *   node features  h      (B, N, H)
@@ -227,6 +228,32 @@ size_t gj_emd_loss_workspace(int32_t batch, int32_t n);
 int gj_emd_loss(int32_t batch, int32_t n, int32_t dim, int32_t coords, const float* p, const float* q, float R, float beta,
                 int32_t flags, float scale, float* terms, float* failed, float* dp, void* workspace, size_t workspace_bytes,
                 void* stream);
+
+/* The Hungarian-matched MSE as a training loss (utils/losses/hungarian_mse/hungarian_mse.py:27-58, losses.HungarianMSELoss): per jet
+ * the coordinate map T of `coords`, the optimal matching of gj_assignment on cost |T(p)_i - T(q)_j|_2, and the squared error of the
+ * reconstruction gathered with the matching, one CTA per jet.  p (B,N,D) is the reconstruction, q (B,N,D) the target, fp32, D in {3,4};
+ * T (losses.hungarian_preprocess, the last three components of p / q taken as (px, py, pz)):
+ *   GJ_HMSE_ABS_CARTESIAN : identity, D' = D;
+ *   GJ_HMSE_ABS_POLAR     : (pt, eta, phi) as losses._to_polar (pt = sqrt(px^2 + py^2 + 1e-16), eta = asinh(pz / (pt + 1e-16)),
+ *                           phi = atan2(py + 1e-16, px + 1e-16)), D' = 3;
+ *   GJ_HMSE_REL_POLAR     : relative to the axis of the TARGET jet (the sum of q's particles, converted the same way):
+ *                           (pt / (pt_jet + 1e-16), eta - eta_jet, phi - phi_jet wrapped into [-pi, pi)), D' = 3;
+ *   GJ_HMSE_REL_CARTESIAN : those relative coordinates as (pt cos phi, pt cos phi, pt sinh eta) (the reference's py), D' = 3.
+ * With sigma = col_for_row of the matching, the loss of jet b is L_b = sum_i |T(p)_sigma(i) - T(q)_i|^2 (fp64 in the workspace).
+ * terms (3) fp32, overwritten: terms[0] = sum_b L_b, terms[1] = 0, terms[2] = scale * terms[0] (the slots of gj_chamfer_fwd_bwd;
+ *   summed in a fixed order, bitwise reproducible).  HungarianMSELoss's mean is scale = 1 / (B N D').
+ * dp (B,N,D) fp32, overwritten: d terms[2] / dp = 2 scale (T(p)_k - T(q)_sigma^-1(k)) J_T(p_k) in p's own coordinates; no gradient
+ *   flows through the matching or the target's axis, and the E component of a 4-vector is 0 except with GJ_HMSE_ABS_CARTESIAN.
+ * col_for_row (B,N) int32, may be NULL: the matching, as gj_assignment returns it for T(p), T(q).
+ * 1 <= N <= 220.  Two launches (the matching and loss, then the sum), no host synchronisation, capturable in a CUDA graph.  Every
+ * argument is checked on the host before any launch; workspace_bytes >= gj_hungarian_mse_loss_workspace(B, N). */
+#define GJ_HMSE_ABS_CARTESIAN 0
+#define GJ_HMSE_ABS_POLAR 1
+#define GJ_HMSE_REL_POLAR 2
+#define GJ_HMSE_REL_CARTESIAN 3
+size_t gj_hungarian_mse_loss_workspace(int32_t batch, int32_t n);
+int gj_hungarian_mse_loss(int32_t batch, int32_t n, int32_t dim, int32_t coords, const float* p, const float* q, float scale,
+                          float* terms, float* dp, int32_t* col_for_row, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Flat fused Adam (torch.optim.Adam defaults: no weight decay, no amsgrad) over n floats.
  * grad_scale multiplies the incoming gradient, l1_lambda*sign(p) and 2*l2_lambda*p are added to it
