@@ -94,6 +94,13 @@ def allreduce_flat_(grad: torch.Tensor, group=None) -> torch.Tensor:
 # --------------------------------------------------------------------------------------------------
 # the fused step
 # --------------------------------------------------------------------------------------------------
+def _with_batch(desc, batch: int):
+    """A copy of a message-passing step descriptor for ``batch`` jets."""
+    d = _lib.MPDesc.from_buffer_copy(desc)
+    d.batch = int(batch)
+    return d
+
+
 def _on_trainer_device(fn):
     """Runs a trainer method with the trainer's GPU as the current device (launchers and streams follow the current device)."""
     import functools
@@ -128,6 +135,17 @@ class GNNAETrainer:
     the global batch (D' = the input width in absolute Cartesian coordinates, else 3).  No gradient flows through the matching.  At
     most 220 particles per jet.
 
+    ``partial_batches`` (default off: every batch has exactly ``batch_size`` jets, and any other size raises) also accepts
+    batches of 1 <= B' < batch_size jets in ``step``, ``step_async``, ``load_batch`` / ``compute_gradients``, ``forward_only`` and
+    ``run_epoch`` (its last batch), such as the tail a ``DataLoader`` without ``drop_last`` yields.  The first batch of a size
+    builds that size's plan: the step descriptors and loss scales of B' (MSE over world B' N D elements, EMD "mean" 1/(world B'),
+    Hungarian 1/(world B' N D')), with every activation, gradient and loss buffer a prefix view of the full-size one; with
+    ``use_cuda_graph`` it also captures that size's graph.  A B'-jet step then returns exactly what a trainer built with
+    ``batch_size=B'`` returns, and allocates no device memory: the workspace, saved and partials buffers are sized at
+    construction for every batch of up to ``batch_size`` jets.  Not with data parallelism: for ``world > 1`` a short batch raises
+    ``NotImplementedError`` -- the mean reductions would need the global jet count, which ranks with different tails only learn
+    through an extra collective.
+
     ``batched_launches`` (default on, used where every step runs the fused tensor-core kernels): the six message-passing steps
     run as a chain -- ONE launch packs all steps' bf16 edge-parameter images, ONE launch reduces all steps' parameter-gradient
     partials (gj_mp_steps_pack / gj_mp_steps_reduce) -- instead of one of each per step; identical results.
@@ -139,7 +157,7 @@ class GNNAETrainer:
                  decoder_metric: str = "euclidean", process_group=None, use_cuda_graph: bool = True,
                  loss_choice: str = "chamfer", polar_coord: bool = False, optimizer: str = "adam",
                  batched_launches: bool = True, emd_loss: Optional[EMDLoss] = None, hungarian_abs_coord: bool = True,
-                 hungarian_polar_coord: bool = False):
+                 hungarian_polar_coord: bool = False, partial_batches: bool = False):
         self.enc, self.dec = encoder, decoder
         g_e, g_d = encoder.encoder, decoder.decoder
         dev = next(encoder.parameters()).device
@@ -196,6 +214,7 @@ class GNNAETrainer:
             raise ValueError(f"Dimension of q ({encoder.input_node_size}) does not match with dimension of p "
                              f"({decoder.output_node_size}), or is not 3 or 4.")
         self.dev, self.B, self.N = dev, int(batch_size), encoder.num_nodes
+        self.batch_size, self.partial_batches = self.B, bool(partial_batches)
         self.lr, self.betas, self.eps = lr, betas, eps
         self.l1, self.l2 = float(l1_lambda), float(l2_lambda)
         self.wc, self.wj = (0.0, 1.0) if chamfer_mode == "reference" else (1.0, float(jet_features_weight))
@@ -264,42 +283,106 @@ class GNNAETrainer:
         if torch.distributed.is_available() and torch.distributed.is_initialized():
             self.world = torch.distributed.get_world_size(process_group)
         if self.loss_choice == "emd":
-            # EMDLoss's reduction over the GLOBAL batch: with "mean" the all-reduced gradient equals the single-device one
-            self.emd_scale = 1.0 if self.emd.reduction == "sum" else 1.0 / (self.world * B)
             self.emd_flags = (_lib.GJ_EMD_NORM if self.emd.norm else 0) | (_lib.GJ_EMD_PERIODIC_PHI if self.emd.periodic_phi else 0)
         if self.loss_choice == "hungarian":
-            # nn.functional.mse_loss's mean over the B N D' elements of the GLOBAL batch, as the MSE branch
-            d_loss = D if self.hmse_coords == _lib.GJ_HMSE_ABS_CARTESIAN else 3
-            self.hmse_scale = 1.0 / (self.world * B * N * d_loss)
+            self.hmse_d = D if self.hmse_coords == _lib.GJ_HMSE_ABS_CARTESIAN else 3
+        self.emd_scale, self.hmse_scale = self._loss_scales(B)
         self.jet_terms = torch.empty((B, 2), **f32)
         # [chamfer | EMD | Hungarian squared error, jet, loss term, sum|p|, sum p^2, EMD jets whose solver hit its cap]
         self.stats = torch.zeros(8, **f32)
         self.stats_host = torch.zeros(8, dtype=torch.float32).pin_memory()
-        ws = max([self.lib.gj_mp_step_bwd_workspace(s["desc"]) for s in self.enc_steps + self.dec_steps] +
-                 [self.lib.gj_mp_step_fwd_workspace(s["desc"]) for s in self.enc_steps + self.dec_steps] +
-                 [self.lib.gj_linear_bwd_workspace(B * N, max(self.latent_w, self.enc_out_w), max(self.h0, self.latent_w)),
-                  self.lib.gj_linear_bwd_workspace(B, max(self.latent_w, N * self.enc_out_w), max(N * self.h0, self.latent_w)),
-                  self.lib.gj_param_norms_workspace(n), self.lib.gj_mse_workspace(), 16] +
-                 ([self.lib.gj_emd_loss_workspace(B, N)] if self.loss_choice == "emd" else []) +
-                 ([self.lib.gj_hungarian_mse_loss_workspace(B, N)] if self.loss_choice == "hungarian" else []))
-        self.ws_bytes = int(ws)
+        all_steps = self.enc_steps + self.dec_steps
+        ws, saved_bytes, pbytes = self._buffer_bytes(B, [s_["desc"] for s_ in all_steps])
+        if self.partial_batches:
+            # every smaller batch runs in these same buffers (_make_plan).  The per-CTA partials follow grids that are not monotonic
+            # in the batch size (a grid capped at a few CTAs per SM evens out its tiles), so a smaller batch can need more than B
+            for b in range(1, B):
+                w, sv, pb = self._buffer_bytes(b, [_with_batch(s_["desc"], b) for s_ in all_steps])
+                ws, saved_bytes, pbytes = max(ws, w), list(map(max, saved_bytes, sv)), list(map(max, pbytes, pb))
+        self.ws_bytes = ws
         self.ws = torch.empty((self.ws_bytes + 3) // 4, **f32)
         # per-step buffers in which the forward call leaves P|Q, the packed edge parameters and the pair distances for the
         # backward call of the same step (0 bytes: that step recomputes them)
-        for st_ in self.enc_steps + self.dec_steps:
-            nbytes = int(self.lib.gj_mp_step_saved_bytes(st_["desc"]))
+        for st_, nbytes in zip(all_steps, saved_bytes):
             st_["saved"] = torch.empty((nbytes + 3) // 4, **f32) if nbytes else None
         # per-chain helper launches (gj_mp_steps_pack / gj_mp_steps_reduce): the packed edge-parameter images of all steps in ONE
         # launch at the start of the forward pass, the parameter-gradient partials of all steps reduced in ONE launch at the end of
         # the backward pass (each step keeps its partials in its own buffer until then) -- where every step supports it
-        all_steps = self.enc_steps + self.dec_steps
-        pbytes = [int(self.lib.gj_mp_step_partials_bytes(s_["desc"])) for s_ in all_steps]
         self.batched = bool(batched_launches) and all(b > 0 for b in pbytes) and all(s_["saved"] is not None for s_ in all_steps)
         for s_, nb in zip(all_steps, pbytes):
             s_["partials"] = torch.empty((nb + 3) // 4, **f32) if self.batched else None
         self.graph = None
         self.use_graph = use_cuda_graph
         self.launches_per_step = None
+        # per batch size: the plan (step descriptors, loss scales, buffers) and its CUDA graph; _use_plan swaps one in
+        self._plans = {B: {k: getattr(self, k) for k in self._PLAN_ATTRS}}
+
+    # what differs between batch sizes: swapped in as attributes, so that the launch sequence reads the resident batch's
+    _PLAN_ATTRS = ("B", "x", "latent", "dlatent", "dec_in", "d_dec_in", "d_enc_out", "dx", "enc_steps", "dec_steps", "recon_raw",
+                   "recon", "dp", "dp_raw", "jet_terms", "emd_scale", "hmse_scale", "graph", "launches_per_step")
+    # batch-major, contiguous: the first B' rows of the full-size buffer are the buffer of a B'-jet batch
+    _PREFIX_ATTRS = ("x", "latent", "dlatent", "dec_in", "d_dec_in", "d_enc_out", "dx", "recon", "dp", "dp_raw", "jet_terms")
+
+    def _loss_scales(self, B):
+        """(EMD, Hungarian MSE) gradient scales of a B-jet batch (None where that loss is not the trainer's)."""
+        emd = hmse = None
+        if self.loss_choice == "emd":
+            # EMDLoss's reduction over the GLOBAL batch: with "mean" the all-reduced gradient equals the single-device one
+            emd = 1.0 if self.emd.reduction == "sum" else 1.0 / (self.world * B)
+        if self.loss_choice == "hungarian":
+            # nn.functional.mse_loss's mean over the B N D' elements of the GLOBAL batch, as the MSE branch
+            hmse = 1.0 / (self.world * B * self.N * self.hmse_d)
+        return emd, hmse
+
+    def _buffer_bytes(self, B, descs):
+        """(workspace, [saved per step], [partials per step]) bytes that a B-jet batch of the steps ``descs`` needs."""
+        lib, N = self.lib, self.N
+        ws = max([lib.gj_mp_step_bwd_workspace(d) for d in descs] + [lib.gj_mp_step_fwd_workspace(d) for d in descs] +
+                 [lib.gj_linear_bwd_workspace(B * N, max(self.latent_w, self.enc_out_w), max(self.h0, self.latent_w)),
+                  lib.gj_linear_bwd_workspace(B, max(self.latent_w, N * self.enc_out_w), max(N * self.h0, self.latent_w)),
+                  lib.gj_param_norms_workspace(self.flat.numel()), lib.gj_mse_workspace(), 16] +
+                 ([lib.gj_emd_loss_workspace(B, N)] if self.loss_choice == "emd" else []) +
+                 ([lib.gj_hungarian_mse_loss_workspace(B, N)] if self.loss_choice == "hungarian" else []))
+        return (int(ws), [int(lib.gj_mp_step_saved_bytes(d)) for d in descs], [int(lib.gj_mp_step_partials_bytes(d)) for d in descs])
+
+    def _make_plan(self, B):
+        """The plan of a batch of B < batch_size jets: the step descriptors and loss scales of B over the full-size memory -- every
+        activation, gradient and loss buffer a prefix view, the workspace, saved and partials buffers shared as they are."""
+        full = self._plans[self.batch_size]
+        plan = {k: full[k][:B] for k in self._PREFIX_ATTRS}
+        steps = lambda ss: [dict(s, desc=_with_batch(s["desc"], B), out=s["out"][:B], e=s["e"][:B],
+                                 din=None if s["din"] is None else s["din"][:B]) for s in ss]
+        plan.update(B=B, enc_steps=steps(full["enc_steps"]), dec_steps=steps(full["dec_steps"]), graph=None, launches_per_step=None)
+        plan["recon_raw"] = plan["dec_steps"][-1]["out"]
+        plan["emd_scale"], plan["hmse_scale"] = self._loss_scales(B)
+        all_steps = plan["enc_steps"] + plan["dec_steps"]
+        ws, saved_bytes, pbytes = self._buffer_bytes(B, [s["desc"] for s in all_steps])
+        have = lambda t: 0 if t is None else 4 * t.numel()
+        if (ws > self.ws_bytes or any(n > have(s["saved"]) for n, s in zip(saved_bytes, all_steps)) or
+                (self.batched and any(n > have(s["partials"]) for n, s in zip(pbytes, all_steps)))):
+            raise RuntimeError(f"internal error: a batch of {B} jets needs larger workspace / saved / partials buffers than the trainer "
+                               f"allocated for batches of up to {self.batch_size} jets")
+        return plan
+
+    def _use_plan(self, B):
+        """Makes the plan of a B-jet batch the resident one (built the first time B appears)."""
+        if B != self.B:
+            plan = self._plans.get(B)
+            if plan is None:
+                plan = self._plans[B] = self._make_plan(B)
+            self.__dict__.update(plan)
+
+    def _jets_in(self, x) -> int:
+        """The number of jets of batch ``x``.  Without ``partial_batches`` it is always ``batch_size``: a batch of another size
+        then fails where it is copied in, as it always has."""
+        if not self.partial_batches or x.numel() == self.batch_size * self.N * self.F:
+            return self.batch_size
+        if x.dim() != 3 or tuple(x.shape[1:]) != (self.N, self.F) or not 1 <= x.shape[0] <= self.batch_size:
+            raise ValueError(f"batch of {tuple(x.shape)}: expected (B', {self.N}, {self.F}) with 1 <= B' <= batch_size = {self.batch_size}")
+        if self.world > 1:
+            raise NotImplementedError("a batch of fewer than batch_size jets with more than one data-parallel rank: the mean reductions "
+                                      "would need the global jet count, which the ranks only learn through an extra collective")
+        return int(x.shape[0])
 
     def _plan_graphnet(self, g, flat_off, in_width, metric):
         steps, off, width_in = [], flat_off, in_width
@@ -468,13 +551,15 @@ class GNNAETrainer:
     @_on_trainer_device
     def forward_only(self, x: torch.Tensor):
         """encoder + decoder forward on a (B,N,F) batch (host or device); returns (latent, recon) device views."""
-        self.x.copy_(x.reshape(self.x.shape), non_blocking=True)
+        self.load_batch(x)
         self._fwd(torch.cuda.current_stream().cuda_stream)
         return self.latent, self.recon
 
     @_on_trainer_device
     def load_batch(self, x: torch.Tensor) -> None:
-        """Host (ideally pinned) or device batch -> the step's resident input buffer."""
+        """Host (ideally pinned) or device batch -> the step's resident input buffer (with ``partial_batches``, a batch of
+        B' < batch_size jets makes the plan of B' the resident one)."""
+        self._use_plan(self._jets_in(x))
         self.x.copy_(x.reshape(self.x.shape), non_blocking=True)
 
     @_on_trainer_device
@@ -495,6 +580,7 @@ class GNNAETrainer:
                 self._fwd_bwd()
             ops.LAUNCHES["count"] -= self.launches_per_step - 1    # the capture pass launched nothing
             self.graph = g
+            self._plans[self.B].update(graph=g, launches_per_step=self.launches_per_step)
         self.graph.replay()
         ops.LAUNCHES["count"] += self.launches_per_step - 1
 
@@ -546,10 +632,12 @@ class GNNAETrainer:
         asynchronous copies into pinned host memory, and the stream is synchronised ONCE at the end of the epoch.
 
         ``loader`` yields (B, N, F) batches (host, ideally pinned, or device) of exactly ``batch_size`` jets (use
-        ``drop_last=True``; the kernels run on fixed shapes).  ``is_train=False`` is the validation pass: forward and loss
-        only, parameters untouched.  Returns ``(epoch_avg_loss, recons_data, target_data, latent_data)`` like the reference:
-        the mean of the batch losses over the batches (train.py:108) and, with ``collect``, the concatenated host tensors
-        (else ``None``).  The host tensors are views of pinned epoch buffers the trainer keeps, one set for training passes and
+        ``drop_last=True``; the kernels run on fixed shapes) -- or, for a trainer built with ``partial_batches=True``, a last
+        batch of fewer jets, as a ``DataLoader`` without ``drop_last`` yields it (a short batch anywhere else raises
+        ``ValueError``).  ``is_train=False`` is the validation pass: forward and loss only, parameters untouched.  Returns
+        ``(epoch_avg_loss, recons_data, target_data, latent_data)`` like the reference: the mean of the batch losses over the
+        batches (train.py:108) and, with ``collect``, the concatenated host tensors of every jet the loader yielded (else
+        ``None``).  The host tensors are views of pinned epoch buffers the trainer keeps, one set for training passes and
         one for validation passes (the reference's train_loop calls train() then validate() and uses both results afterwards,
         utils/train.py:196-236): they stay valid until the next ``run_epoch`` call of the SAME kind (clone them to keep several
         epochs)."""
@@ -564,19 +652,21 @@ class GNNAETrainer:
         # epoch-sized pinned host buffers (allocated once and kept: pinning memory synchronises the device) and device log
         caches = self.__dict__.setdefault("_epoch_buffers", {})      # one set per pass kind: train()'s outputs survive validate()
         cache = caches.get(bool(is_train))
+        full = self._plans[self.batch_size]
         if cache is None or cache["nb"] < nb or (collect and cache["recon"] is None):
             pin = lambda shape: torch.empty((nb,) + tuple(shape), dtype=torch.float32).pin_memory()
             cache = {"nb": nb, "log": torch.zeros((nb, self.stats.numel()), device=self.dev, dtype=torch.float32),
-                     "recon": pin(self.recon.shape) if collect else None, "latent": pin(self.latent.shape) if collect else None,
-                     "target": pin(self.x.shape) if collect else None}
+                     "recon": pin(full["recon"].shape) if collect else None, "latent": pin(full["latent"].shape) if collect else None,
+                     "target": pin(full["x"].shape) if collect else None}
             caches[bool(is_train)] = cache
-        i = 0
+        i = jets = 0
         for x in loader:
             if i >= nb:
                 raise ValueError("run_epoch: the loader yielded more batches than len(loader)")
-            if x.numel() != self.x.numel():
+            if x.numel() != full["x"].numel() and not (self.partial_batches and i == nb - 1):
                 raise ValueError(f"run_epoch: batch of {tuple(x.shape)} does not match the trainer's fixed "
-                                 f"{tuple(self.x.shape)} (drop the last, ragged batch)")
+                                 f"{tuple(full['x'].shape)} (" + ("only the last batch may be short)" if self.partial_batches else
+                                                                  "drop the last, ragged batch)"))
             self.load_batch(x)
             if is_train:
                 self.compute_gradients()
@@ -584,19 +674,20 @@ class GNNAETrainer:
                 self._fwd(st.cuda_stream)
                 self._loss(st.cuda_stream)
             cache["log"][i].copy_(self.stats, non_blocking=True)      # device -> device, stream ordered
-            if collect:
-                cache["recon"][i].copy_(self.recon, non_blocking=True)
-                cache["latent"][i].copy_(self.latent, non_blocking=True)
-                cache["target"][i].copy_(self.x, non_blocking=True)
+            if collect:      # a short last batch fills the first B rows of its slot
+                cache["recon"][i, :self.B].copy_(self.recon, non_blocking=True)
+                cache["latent"][i, :self.B].copy_(self.latent, non_blocking=True)
+                cache["target"][i, :self.B].copy_(self.x, non_blocking=True)
             if is_train:
                 self.apply_gradients()
             i += 1
+            jets += self.B
         log = cache["log"][:i].cpu()                                  # the epoch's one synchronising read
         st.synchronize()
         avg = sum(self.loss_from_stats(row) for row in log) / i
         if not collect:
             return avg, None, None, None
-        flat = lambda t: t[:i].reshape((-1,) + tuple(t.shape[2:]))     # views of the epoch buffers (see the docstring)
+        flat = lambda t: t[:i].reshape((-1,) + tuple(t.shape[2:]))[:jets]     # views of the epoch buffers (see the docstring)
         return avg, flat(cache["recon"]), flat(cache["target"]), flat(cache["latent"])
 
     def flat_gradient(self) -> torch.Tensor:
