@@ -70,6 +70,10 @@ SIGNATURES = {
     "gj_param_norms": (C.c_int, [_P, _SZ, _P, _P, _SZ, _P]),
     "gj_optimizer_step_flat": (C.c_int, [_I, _P, _P, _P, _P, _SZ, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _P]),
     "gj_param_norms_workspace": (_SZ, [_SZ]),
+    "gj_nonfinite_flag": (C.c_int, [_P, _I, _P, _P]),
+    "gj_nonfinite_check": (C.c_int, [_P, _SZ, _P, _P, _P]),
+    "gj_adam_step_flat_guarded": (C.c_int, [_P, _P, _P, _P, _SZ, _F, _F, _F, _F, _P, _P, _F, _F, _F, _P]),
+    "gj_optimizer_step_flat_guarded": (C.c_int, [_I, _P, _P, _P, _P, _SZ, _F, _F, _F, _F, _F, _F, _F, _P, _P, _P]),
     "gj_latent_mean_fwd": (C.c_int, [_I, _I, _I, _P, _P, _P]),
     "gj_latent_mean_bwd": (C.c_int, [_I, _I, _I, _P, _P, _P]),
     "gj_latent_extreme_fwd": (C.c_int, [_I, _I, _I, _I, _P, _P, _P]),

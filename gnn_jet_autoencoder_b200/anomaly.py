@@ -115,10 +115,11 @@ def _emd_polar(x: torch.Tensor, polar_coord: bool) -> torch.Tensor:
 
 
 def _emd_solve(p: torch.Tensor, q: torch.Tensor, R: float, beta: float, norm: bool, periodic_phi: bool, want_flow: bool = False,
-               want_grad: bool = False, want_potentials: bool = False):
+               want_grad: bool = False, want_potentials: bool = False, first: int = 0):
     """One ``gj_emd`` launch on [pt, eta, phi] jets p (B, Np, 3), q (B, Nq, 3): (emd (B,) float64, flow (B, Np, Nq) float64,
-    dEMD/dp (B, Np, 3) float32, potentials (B, Np+1+Nq+1) float64), the last three None unless asked for.  Raises if a jet's
-    solver did not converge."""
+    dEMD/dp (B, Np, 3) float32, potentials (B, Np+1+Nq+1) float64), the last three None unless asked for.  Raises ``ValueError``
+    naming the jets (numbered from ``first``) with a non-finite pt, eta or phi (the solver does not run on them), and ``RuntimeError`` if a jet's solver did
+    not converge."""
     if p.dim() != 3 or q.dim() != 3 or p.shape[0] != q.shape[0] or p.shape[2] != 3 or q.shape[2] != 3:
         raise ValueError(f"expected (B, Np, 3) and (B, Nq, 3) jets, got {tuple(p.shape)} and {tuple(q.shape)}")
     dev = p.device if p.is_cuda else _device()
@@ -136,6 +137,9 @@ def _emd_solve(p: torch.Tensor, q: torch.Tensor, R: float, beta: float, norm: bo
     with torch.cuda.device(dev):
         _lib.check(_lib.load().gj_emd(B, Np, Nq, pc.data_ptr(), qc.data_ptr(), float(R), float(beta), flags, emd.data_ptr(), ptr(flow),
                                       ptr(dp), ptr(pot), status.data_ptr(), None, 0, torch.cuda.current_stream().cuda_stream), "gj_emd")
+    nonfinite = [first + k for k in (status == 2).nonzero().flatten().tolist()]
+    if nonfinite:
+        raise ValueError(f"gj_emd: jet(s) {nonfinite} have a NaN or infinite pt, eta or phi: their EMD is not defined")
     bad = int((status != 0).sum())
     if bad:
         raise RuntimeError(f"gj_emd: the transport solver did not converge for {bad} of {B} jets")
@@ -153,14 +157,15 @@ def emd(p: torch.Tensor, q: torch.Tensor, R: float = 1.0, beta: float = 1.0, nor
     p (B, Np, 3) and q (B, Nq, 3) are [pt, eta, phi] jets, or Cartesian 3- / 4-vectors with ``polar_coord=False``; Np and Nq
     may differ (at most 150 each).  ``norm`` divides each jet's weights by its total.  ``return_flow`` also returns the optimal
     flow (B, Np, Nq) float64.  A positive ``batch_size`` walks the jets in batches and returns CPU tensors, like the other
-    scores here.  Raises if a jet's solver did not converge."""
-    def one(a, b):
+    scores here.  Raises ``ValueError`` naming the jets with a NaN or infinite pt, eta or phi (their EMD is not defined), and
+    ``RuntimeError`` if a jet's solver did not converge."""
+    def one(a, b, first=0):
         dev = a.device if a.is_cuda else _device()
         e, f, _, _ = _emd_solve(_emd_polar(a.to(dev), polar_coord), _emd_polar(b.to(dev), polar_coord), R, beta, norm, periodic_phi,
-                                want_flow=return_flow)
+                                want_flow=return_flow, first=first)
         return e, f
     if batch_size is not None and batch_size > 0 and p.shape[0] > 0:
-        parts = [one(p[i:i + batch_size], q[i:i + batch_size]) for i in range(0, p.shape[0], batch_size)]
+        parts = [one(p[i:i + batch_size], q[i:i + batch_size], i) for i in range(0, p.shape[0], batch_size)]
         e = torch.cat([x[0].cpu() for x in parts])
         f = torch.cat([x[1].cpu() for x in parts]) if return_flow else None
     else:

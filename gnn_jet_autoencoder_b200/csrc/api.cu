@@ -118,6 +118,12 @@ int gj_adam_launch(float*, const float*, float*, float*, size_t, float, float, f
                    cudaStream_t);
 size_t gj_norms_ws_bytes(size_t);
 int gj_optimizer_launch(int, float*, const float*, float*, float*, size_t, float, float, float, float, float, float, float, cudaStream_t);
+int gj_nonfinite_flag_launch(const float*, int, float*, cudaStream_t);
+int gj_nonfinite_check_launch(const float*, size_t, int*, float*, cudaStream_t);
+int gj_adam_guarded_launch(float*, const float*, float*, float*, size_t, float, float, float, float, const int*, int*, float, float, float,
+                           cudaStream_t);
+int gj_optimizer_guarded_launch(int, float*, const float*, float*, float*, size_t, float, float, float, float, float, float, float,
+                                const int*, int*, cudaStream_t);
 int gj_norms_launch(const float*, size_t, float*, void*, size_t, cudaStream_t);
 int gj_latent_mean_fwd_launch(int, int, int, const float*, float*, cudaStream_t);
 int gj_latent_mean_bwd_launch(int, int, int, const float*, float*, cudaStream_t);
@@ -555,6 +561,40 @@ int gj_optimizer_step_flat(int32_t kind, float* param, const float* grad, float*
   if (n && (!param || !grad || !momentum_buf || !sq_acc)) { gj_set_error("gj_optimizer_step_flat: null pointer"); return GJ_ERR_INVALID; }
   return gj_optimizer_launch(kind, param, grad, momentum_buf, sq_acc, n, lr, alpha, momentum, eps, grad_scale, l1_lambda, l2_lambda,
                              (cudaStream_t)stream);
+}
+
+int gj_nonfinite_flag(const float* terms, int32_t count, float* out, void* stream) {
+  g_err[0] = 0;
+  if (count < 0 || count > 64) { gj_set_error("gj_nonfinite_flag: 0 <= count <= 64, got %d", count); return GJ_ERR_INVALID; }
+  if (!out || (count && !terms)) { gj_set_error("gj_nonfinite_flag: null pointer"); return GJ_ERR_INVALID; }
+  return gj_nonfinite_flag_launch(terms, count, out, (cudaStream_t)stream);
+}
+
+int gj_nonfinite_check(const float* x, size_t n, int32_t* skip, float* flag, void* stream) {
+  g_err[0] = 0;
+  if (!skip || (n && !x)) { gj_set_error("gj_nonfinite_check: null pointer"); return GJ_ERR_INVALID; }
+  return gj_nonfinite_check_launch(x, n, skip, flag, (cudaStream_t)stream);
+}
+
+int gj_adam_step_flat_guarded(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr, float beta1,
+                              float beta2, float eps, const int32_t* skip, int32_t* step_state, float grad_scale, float l1_lambda,
+                              float l2_lambda, void* stream) {
+  g_err[0] = 0;
+  if (!skip || !step_state || (n && (!param || !grad || !exp_avg || !exp_avg_sq))) {
+    gj_set_error("gj_adam_step_flat_guarded: null pointer"); return GJ_ERR_INVALID; }
+  return gj_adam_guarded_launch(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, skip, step_state, grad_scale, l1_lambda,
+                                l2_lambda, (cudaStream_t)stream);
+}
+
+int gj_optimizer_step_flat_guarded(int32_t kind, float* param, const float* grad, float* momentum_buf, float* sq_acc, size_t n, float lr,
+                                   float alpha, float momentum, float eps, float grad_scale, float l1_lambda, float l2_lambda,
+                                   const int32_t* skip, int32_t* step_state, void* stream) {
+  g_err[0] = 0;
+  if (kind < GJ_OPT_RMSPROP || kind > GJ_OPT_SGD) { gj_set_error("gj_optimizer_step_flat_guarded: unknown optimiser %d", kind); return GJ_ERR_INVALID; }
+  if (!skip || (n && (!param || !grad || !momentum_buf || !sq_acc))) {
+    gj_set_error("gj_optimizer_step_flat_guarded: null pointer"); return GJ_ERR_INVALID; }
+  return gj_optimizer_guarded_launch(kind, param, grad, momentum_buf, sq_acc, n, lr, alpha, momentum, eps, grad_scale, l1_lambda,
+                                     l2_lambda, skip, step_state, (cudaStream_t)stream);
 }
 
 size_t gj_param_norms_workspace(size_t n) { return gj_norms_ws_bytes(n); }

@@ -143,7 +143,8 @@ __global__ void pair_min_dist_kernel(int np_, int nq, int dim, int lorentz, cons
 // utils/losses/hungarian_mse/hungarian_mse.py:51-56, which call scipy.optimize.linear_sum_assignment jet by jet on the
 // host).  One CTA per jet, thread j owns column j: the O(n^3) shortest-augmenting-path Hungarian method with row / column
 // potentials (u, v), where the scan over the columns of every path step -- relax, arg-min, potential update -- runs across
-// the threads.  Costs are fp32 (|p_i - q_j|_2 or the Lorentz norm squared), potentials and slacks fp64.
+// the threads.  Costs are fp32 (|p_i - q_j|_2 or the Lorentz norm squared), potentials and slacks fp64.  A jet with a cost that is
+// not finite is not solved (identity matching, NaN cost or loss, zero gradient rows): asg_cost checks before asg_solve runs.
 // col_for_row[b][i] = column assigned to row i (linear_sum_assignment's second array for a square matrix).
 constexpr int kAsgMaxParticles = 220;     // the largest n with assignment_smem(n) <= 200 KB
 
@@ -171,19 +172,24 @@ __device__ __forceinline__ AsgState asg_state(int n) {
 }
 
 // cost[i][j] = |sp_i - sq_j|_2 (lorentz: E^2 - px^2 - py^2 - pz^2 of the difference) and the solver's initial state; the staged
-// jets must be visible to the whole CTA (a __syncthreads after the staging)
-__device__ __forceinline__ void asg_cost(const AsgState& S, int n, int lorentz) {
+// jets must be visible to the whole CTA (a __syncthreads after the staging).  Returns, in every thread, whether every cost is finite:
+// the caller must not run asg_solve otherwise -- a NaN or infinite cost never wins a comparison, so the path search would leave
+// stale entries in way[] and its augmentation walk need not end.
+__device__ __forceinline__ bool asg_cost(const AsgState& S, int n, int lorentz) {
   const int tid = threadIdx.x;
   for (int idx = tid; idx <= n; idx += blockDim.x) { S.u[idx] = 0.0; S.prow[idx] = 0; S.way[idx] = 0; }
   const float s1 = lorentz ? -1.f : 1.f;
+  bool finite = true;
   for (int idx = tid; idx < n * n; idx += blockDim.x) {
     const int i = idx / n, j = idx - i * n;
     const float4 a = *reinterpret_cast<const float4*>(S.sp + i * 4), c = *reinterpret_cast<const float4*>(S.sq + j * 4);
     const float dx = a.x - c.x, dy = a.y - c.y, dz = a.z - c.z, dw = a.w - c.w;
     const float d2 = dx * dx + s1 * (dy * dy + dz * dz + dw * dw);
-    S.cost[idx] = lorentz ? d2 : sqrtf(d2);
+    const float cij = lorentz ? d2 : sqrtf(d2);
+    S.cost[idx] = cij;
+    finite &= isfinite(cij);
   }
-  __syncthreads();
+  return !__syncthreads_or(!finite);
 }
 
 // The shortest-augmenting-path solve on S.cost (the whole CTA calls it); leaves the matching in S.prow: prow[j] = 1-based row
@@ -254,7 +260,11 @@ __global__ void assignment_kernel(int n, int dim, int lorentz, const float* __re
     S.sq[idx] = c < dim ? __ldg(qg + r * dim + c) : 0.f;
   }
   __syncthreads();
-  asg_cost(S, n, lorentz);
+  if (!asg_cost(S, n, lorentz)) {      // not solved: identity matching, NaN cost
+    for (int i = tid; i < n; i += blockDim.x) col_for_row[(size_t)b * n + i] = i;
+    if (total_cost && tid == 0) total_cost[b] = __int_as_float(0x7fffffff);
+    return;
+  }
   asg_solve(S, n);
   const int j = tid + 1;
   const bool has_col = j <= n;
@@ -327,7 +337,14 @@ __global__ void hungarian_mse_loss_kernel(int n, int dim, int coords, float scal
     hmse_stage(qg, k, dim, coords, axis, S.sq + k * 4);
   }
   __syncthreads();
-  asg_cost(S, n, 0);
+  if (!asg_cost(S, n, 0)) {      // not solved: identity matching, NaN loss, zero gradient rows
+    for (int k = tid; k < n; k += blockDim.x) {
+      if (col_for_row) col_for_row[(size_t)b * n + k] = k;
+      for (int m = 0; m < dim; ++m) dp[((size_t)b * n + k) * dim + m] = 0.f;
+    }
+    if (tid == 0) jet_loss[b] = __longlong_as_double(0x7ff8000000000000ll);
+    return;
+  }
   asg_solve(S, n);
   // thread k owns particle k of p, matched to particle i = sigma^-1(k) of q
   const int k = tid;

@@ -18,7 +18,8 @@
 // quantity exactly, and the potentials move by min(distance, D).  Costs are fp32 and recomputed from the staged particles
 // (the fp64 flow matrix takes the shared memory: 182 KB at 150 x 150), potentials, flows and the EMD are fp64.
 // Bounded: at most N1 N2 + 4 (N1 + N2) + 64 augmentations (N1 = Np + 1, N2 = Nq + 1) of at most N2 steps each; a jet that
-// hits the cap gets status 1.
+// hits the cap gets status 1, one for which no augmenting path is found status 3 (not seen on finite costs).  A jet with a NaN or
+// infinite staged (pt, eta, phi) never reaches the solver: status 2, EMD NaN, gradient rows 0.
 #include <math.h>
 
 #include "gj_common.cuh"
@@ -41,6 +42,9 @@ __device__ __forceinline__ float emd_pair_cost(float2 a, float2 b, float r, floa
   if (beta == 2.f) return t2 / (r * r);
   return t2 > 0.f ? powf(t2 / (r * r), 0.5f * beta) : 0.f;
 }
+
+// pt, eta and phi of a staged particle are finite (checked before the solver: a NaN cost never enters its comparisons)
+__device__ __forceinline__ bool emd_finite(float pt, float2 ep) { return isfinite(pt) & isfinite(ep.x) & isfinite(ep.y); }
 
 // Per-CTA solver state, carved from the dynamic shared memory (emd_smem bytes).  A kernel stages its jet pair into sp / wa (rows
 // i < Np: (eta, phi) and max(pt, 0); the dummy row Np: (0, 0) and 0) and sq / resb (the same for the columns) and calls emd_solve.
@@ -181,7 +185,7 @@ __device__ double emd_solve(const EmdState& S, int np_, int nq, float r, float b
       __syncthreads();
       if (tid == 0) ctl[0] = 0;
     }
-    if (sink < 0) { if (tid == 0) ctl[1] = 2; break; }
+    if (sink < 0) { if (tid == 0) ctl[1] = 3; break; }
     if (has_col) cpred[j] = pred;
     __syncthreads();
     if (tid == 0) {       // bottleneck of the path sink <- row <- column <- ... <- source row, then augment
@@ -193,7 +197,7 @@ __device__ double emd_solve(const EmdState& S, int np_, int nq, float r, float b
         amt = fmin(amt, flow[(size_t)i * n2 + jj]);
         i = cpred[jj];
       }
-      if (src < 0) ctl[1] = 2;
+      if (src < 0) ctl[1] = 3;
       else {
         jj = sink; i = cpred[jj];
         for (int k = 0; k <= n1 + n2; ++k) {
@@ -270,15 +274,27 @@ __global__ void emd_kernel(int np_, int nq, float r, float beta, int norm, int p
   const int b = blockIdx.x, tid = threadIdx.x;
   const float* pg = p + (size_t)b * np_ * 3;
   const float* qg = q + (size_t)b * nq * 3;
+  bool finite = true;
   for (int i = tid; i < n1; i += blockDim.x) {
     const bool real = i < np_;
+    const float pt = real ? __ldg(pg + i * 3) : 0.f;
     S.sp[i] = real ? make_float2(__ldg(pg + i * 3 + 1), __ldg(pg + i * 3 + 2)) : make_float2(0.f, 0.f);
-    S.wa[i] = real ? fmax((double)__ldg(pg + i * 3), 0.0) : 0.0;
+    S.wa[i] = real ? fmax((double)pt, 0.0) : 0.0;
+    finite &= emd_finite(pt, S.sp[i]);
   }
   for (int j = tid; j < n2; j += blockDim.x) {
     const bool real = j < nq;
+    const float pt = real ? __ldg(qg + j * 3) : 0.f;
     S.sq[j] = real ? make_float2(__ldg(qg + j * 3 + 1), __ldg(qg + j * 3 + 2)) : make_float2(0.f, 0.f);
-    S.resb[j] = real ? fmax((double)__ldg(qg + j * 3), 0.0) : 0.0;
+    S.resb[j] = real ? fmax((double)pt, 0.0) : 0.0;
+    finite &= emd_finite(pt, S.sq[j]);
+  }
+  if (__syncthreads_or(!finite)) {      // not solved: status 2, EMD NaN, no flow, NaN potentials, zero gradient rows
+    if (tid == 0) { emd_out[b] = __longlong_as_double(0x7ff8000000000000ll); if (status_out) status_out[b] = 2; }
+    if (flow_out) for (int idx = tid; idx < np_ * nq; idx += blockDim.x) flow_out[(size_t)b * np_ * nq + idx] = 0.0;
+    if (pot_out) for (int k = tid; k < n1 + n2; k += blockDim.x) pot_out[(size_t)b * (n1 + n2) + k] = __longlong_as_double(0x7ff8000000000000ll);
+    if (dp_out) for (int k = tid; k < np_ * 3; k += blockDim.x) dp_out[(size_t)b * np_ * 3 + k] = 0.f;
+    return;
   }
   const double t = emd_solve(S, np_, nq, r, beta, norm, periodic);
   if (tid == 0) {
@@ -321,12 +337,19 @@ __global__ void emd_loss_kernel(int n, int dim, int cartesian, float r, float be
   const int b = blockIdx.x, tid = threadIdx.x;
   const float* pg = p + (size_t)b * n * dim;
   const float* qg = q + (size_t)b * n * dim;
+  bool finite = true;
   for (int i = tid; i < n1; i += blockDim.x) {
     const bool real = i < n;
     const float3 a = real ? emd_load_polar(pg, i, dim, cartesian) : make_float3(0.f, 0.f, 0.f);
     const float3 c = real ? emd_load_polar(qg, i, dim, cartesian) : make_float3(0.f, 0.f, 0.f);
     S.sp[i] = make_float2(a.y, a.z); S.wa[i] = real ? fmax((double)a.x, 0.0) : 0.0;
     S.sq[i] = make_float2(c.y, c.z); S.resb[i] = real ? fmax((double)c.x, 0.0) : 0.0;
+    finite &= emd_finite(a.x, S.sp[i]) & emd_finite(c.x, S.sq[i]);
+  }
+  if (__syncthreads_or(!finite)) {      // not solved: status 2, EMD NaN, zero gradient rows
+    if (tid == 0) { jet_emd[b] = __longlong_as_double(0x7ff8000000000000ll); jet_status[b] = 2; }
+    if (dp) for (int k = tid; k < n * dim; k += blockDim.x) dp[(size_t)b * n * dim + k] = 0.f;
+    return;
   }
   const double t = emd_solve(S, n, n, r, beta, norm, periodic);
   if (tid == 0) { jet_emd[b] = t; jet_status[b] = S.ctl[1]; }
@@ -349,7 +372,8 @@ __global__ void emd_loss_kernel(int n, int dim, int cartesian, float r, float be
   }
 }
 
-// Fixed-order sum of the per-jet EMDs and count of the jets whose solver stopped without the optimum
+// Fixed-order sum of the per-jet EMDs and count of the jets whose solver stopped without the optimum (a jet with non-finite input,
+// status 2, is not counted: its EMD is NaN and makes the sum NaN)
 __global__ void __launch_bounds__(256) emd_loss_sum_kernel(int batch, float scale, const double* __restrict__ jet_emd,
                                                            const int* __restrict__ jet_status, float* __restrict__ terms,
                                                            float* __restrict__ failed) {
@@ -358,7 +382,7 @@ __global__ void __launch_bounds__(256) emd_loss_sum_kernel(int batch, float scal
   __shared__ int redf[8];
   double s = 0.0;
   int f = 0;
-  for (int b = threadIdx.x; b < batch; b += 256) { s += jet_emd[b]; f += jet_status[b] != 0; }
+  for (int b = threadIdx.x; b < batch; b += 256) { s += jet_emd[b]; f += jet_status[b] != 0 && jet_status[b] != 2; }
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) { s += __shfl_down_sync(0xffffffffu, s, d); f += __shfl_down_sync(0xffffffffu, f, d); }
   if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = s; redf[threadIdx.x >> 5] = f; }

@@ -58,6 +58,118 @@ __global__ void optimizer_kernel(int kind, float* __restrict__ p, const float* _
   }
 }
 
+// ---- the non-finite step guard (GNNAETrainer(nonfinite="skip" | "raise")) ----
+// out[0] = 0 if terms[0..count) are all finite, else NaN.  The trainer writes it into the element past the end of the flat gradient,
+// so that the gradient all-reduce carries a non-finite loss of one rank to every rank, as it carries a non-finite gradient.
+__global__ void nonfinite_flag_kernel(const float* __restrict__ terms, int count, float* __restrict__ out) {
+  gj_pdl_sync();
+  if (threadIdx.x != 0) return;
+  bool ok = true;
+  for (int k = 0; k < count; ++k) ok &= isfinite(terms[k]);
+  out[0] = ok ? 0.f : __int_as_float(0x7fffffff);
+}
+
+// skip[0] = 1 if any of x[0..n) is not finite, else 0; flag[0] (optional) the same as a float.  One CTA: the decision is a few
+// hundred KB at most (the flat gradient of a training step), and one CTA needs no cross-CTA combination.
+constexpr int kCheckThreads = 1024;
+__global__ void __launch_bounds__(kCheckThreads) nonfinite_check_kernel(const float* __restrict__ x, size_t n, int vec,
+                                                                        int* __restrict__ skip, float* __restrict__ flag) {
+  gj_pdl_sync();
+  bool ok = true;
+  size_t i = threadIdx.x;
+  if (vec) {      // 16-byte aligned: float4 reads, four loads in flight per thread
+    const float4* x4 = reinterpret_cast<const float4*>(x);
+    const size_t n4 = n / 4;
+    for (; i + 3 * kCheckThreads < n4; i += 4 * kCheckThreads) {
+      float4 v[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) v[u] = __ldg(x4 + i + (size_t)u * kCheckThreads);
+#pragma unroll
+      for (int u = 0; u < 4; ++u) ok &= isfinite(v[u].x) & isfinite(v[u].y) & isfinite(v[u].z) & isfinite(v[u].w);
+    }
+    for (; i < n4; i += kCheckThreads) { const float4 v = __ldg(x4 + i); ok &= isfinite(v.x) & isfinite(v.y) & isfinite(v.z) & isfinite(v.w); }
+    i = 4 * n4 + threadIdx.x;
+  }
+  for (; i < n; i += kCheckThreads) ok &= isfinite(__ldg(x + i));
+  const int bad = __syncthreads_or(!ok);
+  if (threadIdx.x == 0) {
+    skip[0] = bad;
+    if (flag) flag[0] = bad ? 1.f : 0.f;
+  }
+}
+
+// Called by every CTA of a guarded optimiser launch that applied its update, after its last read of state[0]: the last CTA to
+// arrive advances the applied-step count state[0]; atomicInc wraps the arrival counter state[1] back to 0 for the next launch.
+__device__ __forceinline__ void guard_count_applied(int* state) {
+  __syncthreads();
+  if (threadIdx.x == 0 && atomicInc(reinterpret_cast<unsigned*>(state + 1), gridDim.x - 1) == gridDim.x - 1) state[0] += 1;
+}
+
+// adam_kernel behind the guard: nothing is written when skip[0] != 0; otherwise the update is step state[0] + 1 (bias correction
+// computed as gj_adam_launch computes it on the host) and state[0] advances
+__global__ void adam_guarded_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                    size_t n, float lr, float b1, float b2, float eps, float gscale, float l1, float l2,
+                                    const int* __restrict__ skip, int* state) {
+  gj_pdl_sync();
+  if (*skip) return;
+  __shared__ float coef[2];
+  if (threadIdx.x == 0) {
+    const int step = *(volatile int*)state + 1;
+    const double bc1 = 1.0 - pow((double)b1, (double)step), bc2 = 1.0 - pow((double)b2, (double)step);
+    coef[0] = (float)(lr / bc1); coef[1] = (float)(1.0 / sqrt(bc2));
+  }
+  __syncthreads();
+  const float lr_over_bc1 = coef[0], inv_sqrt_bc2 = coef[1];
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (; i < n; i += stride) {
+    float pi = p[i];
+    float gi = g[i] * gscale;
+    if (l1 != 0.f) gi += l1 * (pi > 0.f ? 1.f : (pi < 0.f ? -1.f : 0.f));
+    if (l2 != 0.f) gi += 2.f * l2 * pi;
+    float mi = b1 * m[i] + (1.f - b1) * gi;
+    float vi = b2 * v[i] + (1.f - b2) * gi * gi;
+    m[i] = mi; v[i] = vi;
+    float denom = sqrtf(vi) * inv_sqrt_bc2 + eps;
+    p[i] = pi - lr_over_bc1 * (mi / denom);
+  }
+  guard_count_applied(state);
+}
+
+// optimizer_kernel behind the guard (state, optional: the count of applied updates)
+__global__ void optimizer_guarded_kernel(int kind, float* __restrict__ p, const float* __restrict__ g, float* __restrict__ buf,
+                                         float* __restrict__ acc, size_t n, float lr, float alpha, float momentum, float eps,
+                                         float gscale, float l1, float l2, const int* __restrict__ skip, int* state) {
+  gj_pdl_sync();
+  if (*skip) return;
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (; i < n; i += stride) {
+    const float pi = p[i];
+    float gi = g[i] * gscale;
+    if (l1 != 0.f) gi += l1 * (pi > 0.f ? 1.f : (pi < 0.f ? -1.f : 0.f));
+    if (l2 != 0.f) gi += 2.f * l2 * pi;
+    float upd;
+    if (kind == 1) {
+      const float sq = alpha * acc[i] + (1.f - alpha) * gi * gi;
+      acc[i] = sq;
+      const float b = momentum * buf[i] + gi / (sqrtf(sq) + eps);
+      buf[i] = b;
+      upd = b;
+    } else if (kind == 2) {
+      const float sq = acc[i] + gi * gi;
+      acc[i] = sq;
+      upd = gi / (sqrtf(sq) + eps);
+    } else {
+      const float b = momentum * buf[i] + gi;
+      buf[i] = b;
+      upd = b;
+    }
+    p[i] = pi - lr * upd;
+  }
+  if (state) guard_count_applied(state);
+}
+
 __global__ void norms_stage1(const float* __restrict__ p, size_t n, float* __restrict__ part) {
   gj_pdl_sync();
   __shared__ float red[2][8];
@@ -244,6 +356,43 @@ int gj_optimizer_launch(int kind, float* param, const float* grad, float* buf, f
   gj_launch(optimizer_kernel, blocks, 256, 0, stream, kind, param, grad, buf, acc, n, lr, alpha, momentum, eps, gscale, l1, l2);
   cudaError_t ce = cudaGetLastError();
   if (ce != cudaSuccess) { gj_set_error("optimizer launch: %s", cudaGetErrorString(ce)); return GJ_ERR_CUDA; }
+  return GJ_OK;
+}
+
+int gj_nonfinite_flag_launch(const float* terms, int count, float* out, cudaStream_t stream) {
+  gj_launch(nonfinite_flag_kernel, 1, 32, 0, stream, terms, count, out);
+  cudaError_t ce = cudaGetLastError();
+  if (ce != cudaSuccess) { gj_set_error("nonfinite_flag launch: %s", cudaGetErrorString(ce)); return GJ_ERR_CUDA; }
+  return GJ_OK;
+}
+
+int gj_nonfinite_check_launch(const float* x, size_t n, int* skip, float* flag, cudaStream_t stream) {
+  const int vec = ((uintptr_t)x & 15) == 0;
+  gj_launch(nonfinite_check_kernel, 1, kCheckThreads, 0, stream, x, n, vec, skip, flag);
+  cudaError_t ce = cudaGetLastError();
+  if (ce != cudaSuccess) { gj_set_error("nonfinite_check launch: %s", cudaGetErrorString(ce)); return GJ_ERR_CUDA; }
+  return GJ_OK;
+}
+
+int gj_adam_guarded_launch(float* param, const float* grad, float* m, float* v, size_t n, float lr, float b1, float b2, float eps,
+                           const int* skip, int* state, float gscale, float l1, float l2, cudaStream_t stream) {
+  if (n == 0) return GJ_OK;
+  int blocks = (int)((n + 255) / 256); if (blocks > 148 * 8) blocks = 148 * 8;
+  gj_launch(adam_guarded_kernel, blocks, 256, 0, stream, param, grad, m, v, n, lr, b1, b2, eps, gscale, l1, l2, skip, state);
+  cudaError_t ce = cudaGetLastError();
+  if (ce != cudaSuccess) { gj_set_error("guarded adam launch: %s", cudaGetErrorString(ce)); return GJ_ERR_CUDA; }
+  return GJ_OK;
+}
+
+int gj_optimizer_guarded_launch(int kind, float* param, const float* grad, float* buf, float* acc, size_t n, float lr, float alpha,
+                                float momentum, float eps, float gscale, float l1, float l2, const int* skip, int* state,
+                                cudaStream_t stream) {
+  if (n == 0) return GJ_OK;
+  int blocks = (int)((n + 255) / 256); if (blocks > 148 * 8) blocks = 148 * 8;
+  gj_launch(optimizer_guarded_kernel, blocks, 256, 0, stream, kind, param, grad, buf, acc, n, lr, alpha, momentum, eps, gscale, l1, l2,
+            skip, state);
+  cudaError_t ce = cudaGetLastError();
+  if (ce != cudaSuccess) { gj_set_error("guarded optimizer launch: %s", cudaGetErrorString(ce)); return GJ_ERR_CUDA; }
   return GJ_OK;
 }
 

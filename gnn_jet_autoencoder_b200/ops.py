@@ -423,6 +423,12 @@ def set_deterministic(on: bool) -> bool:
 OPTIMIZERS = {"rmsprop": 1, "adagrad": 2, "sgd": 3}
 
 
+def _optimizer_hparams(kind: str):
+    """(kind id, (alpha, momentum, eps)) of the hyper-parameters utils/initialize.py:154-170 passes."""
+    k = OPTIMIZERS[kind.lower()]
+    return k, ((0.99, 0.9, 1e-16) if k == 1 else ((0.0, 0.0, 1e-16) if k == 2 else (0.0, 0.9, 0.0)))
+
+
 @_on_device
 def optimizer_step_flat_(kind: str, param: Tensor, grad: Tensor, momentum_buf: Tensor, sq_acc: Tensor, lr: float = 1e-5,
                          grad_scale: float = 1.0, l1_lambda: float = 0.0, l2_lambda: float = 0.0) -> None:
@@ -431,11 +437,77 @@ def optimizer_step_flat_(kind: str, param: Tensor, grad: Tensor, momentum_buf: T
     for t, n in ((param, "param"), (grad, "grad"), (momentum_buf, "momentum_buf"), (sq_acc, "sq_acc")):
         if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous():
             raise _lib.GnnJetError(f"{n} must be a contiguous float32 CUDA tensor")
-    k = OPTIMIZERS[kind.lower()]
-    alpha, momentum, eps = (0.99, 0.9, 1e-16) if k == 1 else ((0.0, 0.0, 1e-16) if k == 2 else (0.0, 0.9, 0.0))
+    k, (alpha, momentum, eps) = _optimizer_hparams(kind)
     _lib.check(_lib.load().gj_optimizer_step_flat(k, param.data_ptr(), grad.data_ptr(), momentum_buf.data_ptr(), sq_acc.data_ptr(),
                                                   param.numel(), lr, alpha, momentum, eps, grad_scale, l1_lambda, l2_lambda, _stream()),
                "gj_optimizer_step_flat")
+    LAUNCHES["count"] += 1
+
+
+# ---- non-finite step guard (include/gnnjet_b200.h: gj_nonfinite_flag / gj_nonfinite_check / gj_*_step_flat_guarded) ----------
+def _req_i32(t: Tensor, name: str, n: int) -> None:
+    if not t.is_cuda or t.dtype != torch.int32 or not t.is_contiguous() or t.numel() < n:
+        raise _lib.GnnJetError(f"{name} must be a contiguous int32 CUDA tensor of at least {n} elements")
+
+
+def _req_f32(t: Tensor, name: str) -> None:
+    if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous():
+        raise _lib.GnnJetError(f"{name} must be a contiguous float32 CUDA tensor")
+
+
+@_on_device
+def nonfinite_flag_(terms: Tensor, out: Tensor) -> None:
+    """out[0] = 0 if every element of ``terms`` (at most 64) is finite, else NaN: one launch, no host synchronisation."""
+    _req_f32(terms, "terms")
+    _req_f32(out, "out")
+    _lib.check(_lib.load().gj_nonfinite_flag(terms.data_ptr(), terms.numel(), out.data_ptr(), _stream()), "gj_nonfinite_flag")
+    LAUNCHES["count"] += 1
+
+
+@_on_device
+def nonfinite_check_(x: Tensor, skip: Tensor, flag: Tensor | None = None) -> None:
+    """skip[0] = 1 if any element of ``x`` is not finite, else 0 (int32); ``flag[0]`` the same as 1.0 / 0.0: one launch, one CTA, no
+    host synchronisation."""
+    _req_f32(x, "x")
+    _req_i32(skip, "skip", 1)
+    if flag is not None:
+        _req_f32(flag, "flag")
+    _lib.check(_lib.load().gj_nonfinite_check(x.data_ptr(), x.numel(), skip.data_ptr(), _ptr(flag), _stream()), "gj_nonfinite_check")
+    LAUNCHES["count"] += 1
+
+
+@_on_device
+def adam_step_flat_guarded_(param: Tensor, grad: Tensor, exp_avg: Tensor, exp_avg_sq: Tensor, skip: Tensor, step_state: Tensor,
+                            lr: float = 1e-5, betas=(0.9, 0.999), eps: float = 1e-8, grad_scale: float = 1.0, l1_lambda: float = 0.0,
+                            l2_lambda: float = 0.0) -> None:
+    """``adam_step_flat_`` behind the device flag ``skip[0]`` (int32): nothing is written when it is set.  The step number is
+    ``step_state[0] + 1`` (int32, two elements, zero-initialised; ``step_state[0]`` counts the updates applied and the launch advances
+    it when it applies its update, ``step_state[1]`` is the kernel's arrival counter and stays 0)."""
+    for t, n in ((param, "param"), (grad, "grad"), (exp_avg, "exp_avg"), (exp_avg_sq, "exp_avg_sq")):
+        _req_f32(t, n)
+    _req_i32(skip, "skip", 1)
+    _req_i32(step_state, "step_state", 2)
+    _lib.check(_lib.load().gj_adam_step_flat_guarded(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
+                                                     param.numel(), lr, betas[0], betas[1], eps, skip.data_ptr(), step_state.data_ptr(),
+                                                     grad_scale, l1_lambda, l2_lambda, _stream()), "gj_adam_step_flat_guarded")
+    LAUNCHES["count"] += 1
+
+
+@_on_device
+def optimizer_step_flat_guarded_(kind: str, param: Tensor, grad: Tensor, momentum_buf: Tensor, sq_acc: Tensor, skip: Tensor,
+                                 step_state: Tensor | None = None, lr: float = 1e-5, grad_scale: float = 1.0, l1_lambda: float = 0.0,
+                                 l2_lambda: float = 0.0) -> None:
+    """``optimizer_step_flat_`` behind the device flag ``skip[0]``; ``step_state`` (optional, as for ``adam_step_flat_guarded_``)
+    counts the updates applied."""
+    for t, n in ((param, "param"), (grad, "grad"), (momentum_buf, "momentum_buf"), (sq_acc, "sq_acc")):
+        _req_f32(t, n)
+    _req_i32(skip, "skip", 1)
+    if step_state is not None:
+        _req_i32(step_state, "step_state", 2)
+    k, (alpha, momentum, eps) = _optimizer_hparams(kind)
+    _lib.check(_lib.load().gj_optimizer_step_flat_guarded(k, param.data_ptr(), grad.data_ptr(), momentum_buf.data_ptr(), sq_acc.data_ptr(),
+                                                          param.numel(), lr, alpha, momentum, eps, grad_scale, l1_lambda, l2_lambda,
+                                                          skip.data_ptr(), _ptr(step_state), _stream()), "gj_optimizer_step_flat_guarded")
     LAUNCHES["count"] += 1
 
 

@@ -83,6 +83,17 @@ def layout_size(layout) -> int:
     return sum(int(np.prod(s)) for _, s in layout.values())
 
 
+NONFINITE_MODES = ("ignore", "skip", "raise")
+
+
+def nonfinite_mode(value) -> str:
+    """The ``nonfinite`` keyword of GNNAETrainer, checked: 'ignore', 'skip' or 'raise'."""
+    mode = str(value).lower()
+    if mode not in NONFINITE_MODES:
+        raise ValueError(f"nonfinite must be one of {NONFINITE_MODES}, got {value!r}")
+    return mode
+
+
 def allreduce_flat_(grad: torch.Tensor, group=None) -> torch.Tensor:
     """The path's only collective: sum the flat gradient buffer over the data-parallel ranks."""
     import torch.distributed as dist
@@ -149,6 +160,22 @@ class GNNAETrainer:
     ``batched_launches`` (default on, used where every step runs the fused tensor-core kernels): the six message-passing steps
     run as a chain -- ONE launch packs all steps' bf16 edge-parameter images, ONE launch reduces all steps' parameter-gradient
     partials (gj_mp_steps_pack / gj_mp_steps_reduce) -- instead of one of each per step; identical results.
+
+    ``nonfinite`` guards the parameters against a step whose loss or gradient is not finite (the reference's
+    ``torch.autograd.set_detect_anomaly(True)``, train.py:149), on the device and without a host synchronisation:
+      * "ignore" (default): no check; the launches and results of a trainer without the keyword.
+      * "skip": the step's captured graph ends with one launch that writes 0, or NaN if this rank's loss terms are not finite, into an
+        element past the end of the flat gradient (``grad_buffer``, n + 1 floats; ``grad`` and the parameters' ``.grad`` stay the n-float
+        views); after the all-reduce one launch checks the n + 1 summed floats and the optimiser update is skipped on every rank if one
+        is not finite: parameters, moments and the device-resident step counter of Adam's bias correction stay as they were.  The
+        decision is logged in slot 6 of ``stats``.  ``step`` then returns the non-finite loss and counts the step in
+        ``nonfinite_steps``; ``run_epoch`` returns the mean over the batches whose update was applied, sets ``last_epoch_nonfinite``
+        to the indices of the skipped batches (its outputs still hold every jet) and raises ``FloatingPointError`` if every batch was
+        skipped.  A validation pass only records the batches whose loss is not finite in ``last_epoch_nonfinite``.
+      * "raise": "skip", then ``FloatingPointError`` at the host read: right away in ``step``, at the end of the epoch in
+        ``run_epoch`` (naming the skipped batches).  The trainer's state is that before the failing step(s), so the caller can recover.
+    ``step_count`` counts the ``apply_gradients`` calls; ``applied_steps`` (a synchronising read) the updates applied.  Two launches
+    per step more than "ignore".
     """
 
     def __init__(self, encoder, decoder, batch_size: int, *, lr: float = 1e-5, betas=(0.9, 0.999), eps: float = 1e-8,
@@ -157,7 +184,9 @@ class GNNAETrainer:
                  decoder_metric: str = "euclidean", process_group=None, use_cuda_graph: bool = True,
                  loss_choice: str = "chamfer", polar_coord: bool = False, optimizer: str = "adam",
                  batched_launches: bool = True, emd_loss: Optional[EMDLoss] = None, hungarian_abs_coord: bool = True,
-                 hungarian_polar_coord: bool = False, partial_batches: bool = False):
+                 hungarian_polar_coord: bool = False, partial_batches: bool = False, nonfinite: str = "ignore"):
+        self.nonfinite = nonfinite_mode(nonfinite)
+        self.guarded = self.nonfinite != "ignore"
         self.enc, self.dec = encoder, decoder
         g_e, g_d = encoder.encoder, decoder.decoder
         dev = next(encoder.parameters()).device
@@ -227,7 +256,12 @@ class GNNAETrainer:
         self.layout = flat_layout(encoder, decoder)
         n = layout_size(self.layout)
         self.flat = torch.empty(n, device=dev, dtype=torch.float32)
-        self.grad = torch.zeros(n, device=dev, dtype=torch.float32)
+        # with the guard, one float more: this rank's non-finite-loss flag, all-reduced with the gradient (apply_gradients)
+        self.grad_buffer = torch.zeros(n + int(self.guarded), device=dev, dtype=torch.float32)
+        self.grad = self.grad_buffer[:n]
+        # [skip flag of the last decision, optimiser updates applied, the guarded optimisers' arrival counter]
+        self.guard = torch.zeros(3, device=dev, dtype=torch.int32) if self.guarded else None
+        self.nonfinite_steps, self.last_epoch_nonfinite = 0, []
         self.exp_avg = torch.zeros(n, device=dev, dtype=torch.float32)
         self.exp_avg_sq = torch.zeros(n, device=dev, dtype=torch.float32)
         named = OrderedDict([("encoder." + k, p) for k, p in encoder.named_parameters()] +
@@ -288,7 +322,8 @@ class GNNAETrainer:
             self.hmse_d = D if self.hmse_coords == _lib.GJ_HMSE_ABS_CARTESIAN else 3
         self.emd_scale, self.hmse_scale = self._loss_scales(B)
         self.jet_terms = torch.empty((B, 2), **f32)
-        # [chamfer | EMD | Hungarian squared error, jet, loss term, sum|p|, sum p^2, EMD jets whose solver hit its cap]
+        # [chamfer | EMD | Hungarian squared error, jet, loss term, sum|p|, sum p^2, EMD jets whose solver hit its cap,
+        #  1 if the non-finite guard skipped the step's update (validation: if the loss terms are not finite)]
         self.stats = torch.zeros(8, **f32)
         self.stats_host = torch.zeros(8, dtype=torch.float32).pin_memory()
         all_steps = self.enc_steps + self.dec_steps
@@ -541,6 +576,9 @@ class GNNAETrainer:
             steps = self.enc_steps + self.dec_steps
             ops.raw_mp_reduce_steps([s["desc"] for s in steps], [s["partials"].data_ptr() for s in steps],
                                     [G + 4 * s["off"] for s in steps], st)
+        if self.guarded:      # this rank's loss terms -> 0 / NaN past the end of the gradient, summed over the ranks with it
+            _lib.check(lib.gj_nonfinite_flag(self.stats.data_ptr(), 3, G + 4 * self.grad.numel(), st), "nonfinite flag")
+            ops.LAUNCHES["count"] += 1
 
     def _fwd_bwd(self):
         st = torch.cuda.current_stream().cuda_stream
@@ -571,23 +609,43 @@ class GNNAETrainer:
         if self.graph is None:
             before = ops.LAUNCHES["count"]
             self._fwd_bwd()                      # eager warm-up: loads the kernels outside the capture
-            self.launches_per_step = ops.LAUNCHES["count"] - before + 1   # + Adam
+            self.launches_per_step = ops.LAUNCHES["count"] - before + self._apply_launches   # + the optimiser (and the decision)
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
             # thread-local capture mode: other threads of the process (NCCL's watchdog, a pinned-memory loader) may call into the CUDA
             # runtime while the step is being captured; in the default global mode such a call invalidates a long capture
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
                 self._fwd_bwd()
-            ops.LAUNCHES["count"] -= self.launches_per_step - 1    # the capture pass launched nothing
+            ops.LAUNCHES["count"] -= self.launches_per_step - self._apply_launches    # the capture pass launched nothing
             self.graph = g
             self._plans[self.B].update(graph=g, launches_per_step=self.launches_per_step)
         self.graph.replay()
-        ops.LAUNCHES["count"] += self.launches_per_step - 1
+        ops.LAUNCHES["count"] += self.launches_per_step - self._apply_launches
+
+    @property
+    def _apply_launches(self) -> int:
+        """Launches of ``apply_gradients``: the optimiser, and the non-finite decision with the guard."""
+        return 2 if self.guarded else 1
+
+    @property
+    def applied_steps(self) -> int:
+        """The optimiser updates applied so far: ``step_count`` less the steps the non-finite guard skipped.  With
+        ``nonfinite="skip"`` / ``"raise"`` this reads the device counter and so synchronises with the device."""
+        return int(self.guard[1].item()) if self.guarded else self.step_count
 
     @_on_trainer_device
     def apply_gradients(self) -> None:
-        allreduce_flat_(self.grad, self.group)
+        allreduce_flat_(self.grad_buffer, self.group)
         self.step_count += 1
+        if self.guarded:      # the decision over the summed gradient and flags (the same on every rank), then the guarded update
+            ops.nonfinite_check_(self.grad_buffer, self.guard[:1], self.stats[6:7])
+            if self.optimizer == "adam":
+                ops.adam_step_flat_guarded_(self.flat, self.grad, self.exp_avg, self.exp_avg_sq, self.guard[:1], self.guard[1:],
+                                            self.lr, self.betas, self.eps, 1.0, self.l1, self.l2)
+            else:
+                ops.optimizer_step_flat_guarded_(self.optimizer, self.flat, self.grad, self.exp_avg, self.exp_avg_sq, self.guard[:1],
+                                                 self.guard[1:], self.lr, 1.0, self.l1, self.l2)
+            return
         if self.optimizer == "adam":
             ops.adam_step_flat_(self.flat, self.grad, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr, self.betas,
                                 self.eps, 1.0, self.l1, self.l2)
@@ -598,8 +656,8 @@ class GNNAETrainer:
     def step_async(self, x: torch.Tensor) -> None:
         self.load_batch(x)
         self.compute_gradients()
-        self.stats_host.copy_(self.stats, non_blocking=True)
         self.apply_gradients()
+        self.stats_host.copy_(self.stats, non_blocking=True)      # after the non-finite decision, which apply_gradients logs
 
     def loss_from_stats(self, stats) -> float:
         """train.py:376-384: batch loss = loss value + l1_lambda * sum|p| + l2_lambda * sum p^2 (this rank's shard).
@@ -619,9 +677,15 @@ class GNNAETrainer:
 
     @_on_trainer_device
     def step(self, x: torch.Tensor) -> float:
-        """One optimisation step; returns this rank's batch loss (a device->host read, like train.py:77)."""
+        """One optimisation step; returns this rank's batch loss (a device->host read, like train.py:77).  With ``nonfinite`` a
+        skipped step returns its non-finite loss ("skip") or raises ``FloatingPointError`` ("raise")."""
         self.step_async(x)
         torch.cuda.current_stream().synchronize()
+        if self.guarded and float(self.stats_host[6]) != 0:
+            self.nonfinite_steps += 1
+            if self.nonfinite == "raise":
+                raise FloatingPointError("non-finite loss or gradient: the update of this step was skipped, the parameters and the "
+                                         "optimiser state are those before the step")
         return self.loss_from_stats(self.stats_host)
 
     @_on_trainer_device
@@ -636,7 +700,8 @@ class GNNAETrainer:
         batch of fewer jets, as a ``DataLoader`` without ``drop_last`` yields it (a short batch anywhere else raises
         ``ValueError``).  ``is_train=False`` is the validation pass: forward and loss only, parameters untouched.  Returns
         ``(epoch_avg_loss, recons_data, target_data, latent_data)`` like the reference: the mean of the batch losses over the
-        batches (train.py:108) and, with ``collect``, the concatenated host tensors of every jet the loader yielded (else
+        batches (train.py:108; with ``nonfinite="skip"``, over the batches whose update was applied) and, with ``collect``, the
+        concatenated host tensors of every jet the loader yielded (else
         ``None``).  The host tensors are views of pinned epoch buffers the trainer keeps, one set for training passes and
         one for validation passes (the reference's train_loop calls train() then validate() and uses both results afterwards,
         utils/train.py:196-236): they stay valid until the next ``run_epoch`` call of the SAME kind (clone them to keep several
@@ -673,18 +738,30 @@ class GNNAETrainer:
             else:
                 self._fwd(st.cuda_stream)
                 self._loss(st.cuda_stream)
-            cache["log"][i].copy_(self.stats, non_blocking=True)      # device -> device, stream ordered
+                if self.guarded:      # no update to skip: only the flag of the loss terms
+                    ops.nonfinite_check_(self.stats[:3], self.guard[:1], self.stats[6:7])
             if collect:      # a short last batch fills the first B rows of its slot
                 cache["recon"][i, :self.B].copy_(self.recon, non_blocking=True)
                 cache["latent"][i, :self.B].copy_(self.latent, non_blocking=True)
                 cache["target"][i, :self.B].copy_(self.x, non_blocking=True)
             if is_train:
                 self.apply_gradients()
+            cache["log"][i].copy_(self.stats, non_blocking=True)      # device -> device, stream ordered, after the decision
             i += 1
             jets += self.B
         log = cache["log"][:i].cpu()                                  # the epoch's one synchronising read
         st.synchronize()
-        avg = sum(self.loss_from_stats(row) for row in log) / i
+        rows = log
+        if self.guarded:
+            self.last_epoch_nonfinite = [k for k in range(i) if float(log[k, 6]) != 0]
+            if is_train and self.last_epoch_nonfinite:
+                self.nonfinite_steps += len(self.last_epoch_nonfinite)
+                if self.nonfinite == "raise" or len(self.last_epoch_nonfinite) == i:
+                    raise FloatingPointError(f"run_epoch: non-finite loss or gradient in batch(es) {self.last_epoch_nonfinite} of {i}: "
+                                             "their updates were skipped")
+                skipped = set(self.last_epoch_nonfinite)
+                rows = [row for k, row in enumerate(log) if k not in skipped]
+        avg = sum(self.loss_from_stats(row) for row in rows) / len(rows)
         if not collect:
             return avg, None, None, None
         flat = lambda t: t[:i].reshape((-1,) + tuple(t.shape[2:]))[:jets]     # views of the epoch buffers (see the docstring)

@@ -23,6 +23,8 @@
  *   gj_mse_fwd_bwd                   : utils/train.py:359-361 (nn.MSELoss branch of get_loss)
  *   gj_emd_loss                      : the emd branch of get_loss (utils/train.py:330-385) on utils/losses/emd_loss.py
  *   gj_hungarian_mse_loss            : utils/losses/hungarian_mse/hungarian_mse.py:27-58 as a training loss
+ *   gj_nonfinite_flag / _check,      : torch.autograd.set_detect_anomaly(True) of train.py:149, as a device-side skip of a
+ *   gj_*_step_flat_guarded             step whose loss or gradient is not finite
  *
  * Tensor layouts: all tensors are dense row-major float32 in HBM.
  *   node features  h      (B, N, H)
@@ -175,7 +177,9 @@ int gj_pair_min_dist(int32_t batch, int32_t np_, int32_t nq, int32_t dim, int32_
  * utils/losses/hungarian_mse/hungarian_mse.py:51-56, which call scipy.optimize.linear_sum_assignment jet by jet on the host.
  * cost(i, j) = |p_i - q_j|_2 (lorentz == 0) or E^2 - px^2 - py^2 - pz^2 of p_i - q_j (lorentz == 1, D == 4).
  * col_for_row (B,N) int32: column (particle of q) assigned to row i (particle of p) -- linear_sum_assignment(cost)[1];
- * total_cost (B), may be NULL: the assignment's cost.  N <= 220 (the cost matrix lives in shared memory). */
+ * total_cost (B), may be NULL: the assignment's cost.  N <= 220 (the cost matrix lives in shared memory).
+ * A jet with a cost that is not finite (a NaN or infinite coordinate, or a distance that overflows fp32) is not solved: identity
+ * matching, total_cost NaN. */
 int gj_assignment(int32_t batch, int32_t n, int32_t dim, int32_t lorentz, const float* p, const float* q,
                   int32_t* col_for_row, float* total_cost, void* stream);
 
@@ -198,7 +202,9 @@ int gj_assignment(int32_t batch, int32_t n, int32_t dim, int32_t lorentz, const 
  *   potentials_out (B, Np+1+Nq+1) fp64: optimal duals (u_0..u_Np, v_0..v_Nq) of the balanced problem, u_i + v_j <= c_ij with
  *     equality where flow moves, and sum_i a_i u_i + sum_j b_j v_j = EMD;
  *   status_out (B) int32: 0 converged, 1 augmentation cap N1 N2 + 4 (N1 + N2) + 64 reached, N1 = Np + 1, N2 = Nq + 1
- *     (emd_out is then not optimal).
+ *     (emd_out is then not optimal), 2 non-finite input, 3 no augmenting path found (does not occur on finite costs).
+ * A jet with a NaN or infinite pt, eta or phi on either side is not solved (status 2): its EMD is NaN, its flow 0, its potentials NaN
+ * and its dp rows 0.  The check runs before the solver, whose loops are bounded in any case (the cap above).
  * gj_emd_workspace returns 0 for every shape (the solver's state lives in shared memory): workspace may be NULL. */
 #define GJ_EMD_NORM 1
 #define GJ_EMD_PERIODIC_PHI 2
@@ -218,6 +224,8 @@ int gj_emd(int32_t batch, int32_t np_, int32_t nq, const float* p, const float* 
  * terms (3) fp32, overwritten: terms[0] = sum_b EMD_b, terms[1] = 0, terms[2] = scale * terms[0] (the slots of gj_chamfer_fwd_bwd);
  *   the per-jet EMDs are fp64 in the workspace and summed in a fixed order (bitwise reproducible).
  * failed (1) fp32, overwritten: number of jets whose solver stopped at the augmentation cap (their EMD and gradient are not optimal).
+ *   A jet with a non-finite (pt, eta, phi) on either side (after the conversion) is not solved and not counted here: its EMD is NaN,
+ *   so terms are NaN, and its dp rows are 0.
  * dp (B,N,D) fp32, may be NULL: scale * dEMD_b/dp as gj_emd's dp_out (rounded to fp32 first), through the Jacobian of the
  *   conversion in Cartesian coordinates; the E component is 0.
  * Two launches (the solver, then the sum), no host synchronisation, capturable in a CUDA graph.  Every argument is checked on the
@@ -245,6 +253,8 @@ int gj_emd_loss(int32_t batch, int32_t n, int32_t dim, int32_t coords, const flo
  * dp (B,N,D) fp32, overwritten: d terms[2] / dp = 2 scale (T(p)_k - T(q)_sigma^-1(k)) J_T(p_k) in p's own coordinates; no gradient
  *   flows through the matching or the target's axis, and the E component of a 4-vector is 0 except with GJ_HMSE_ABS_CARTESIAN.
  * col_for_row (B,N) int32, may be NULL: the matching, as gj_assignment returns it for T(p), T(q).
+ * A jet with a cost that is not finite (as for gj_assignment, on T(p), T(q)) is not solved: identity matching, L_b NaN (so terms are
+ * NaN), dp rows 0.
  * 1 <= N <= 220.  Two launches (the matching and loss, then the sum), no host synchronisation, capturable in a CUDA graph.  Every
  * argument is checked on the host before any launch; workspace_bytes >= gj_hungarian_mse_loss_workspace(B, N). */
 #define GJ_HMSE_ABS_CARTESIAN 0
@@ -271,6 +281,32 @@ int gj_adam_step_flat(float* param, const float* grad, float* exp_avg, float* ex
 #define GJ_OPT_SGD 3
 int gj_optimizer_step_flat(int32_t kind, float* param, const float* grad, float* momentum_buf, float* sq_acc, size_t n, float lr,
                            float alpha, float momentum, float eps, float grad_scale, float l1_lambda, float l2_lambda, void* stream);
+
+/* Non-finite step guard: a training step whose loss or gradient is not finite skips its optimiser update on the device, without a
+ * host synchronisation (GNNAETrainer(nonfinite="skip" | "raise"); the analogue of torch.autograd.set_detect_anomaly with the
+ * parameters and optimiser state kept as they were before the step).  Sequence of one data-parallel step:
+ *   gj_nonfinite_flag     : one launch, out[0] = 0 if terms[0..count) are all finite, else NaN (count <= 64).  The trainer points out
+ *                           at one element past the end of the flat gradient (a buffer of n + 1 floats), so that the gradient's
+ *                           all-reduce(sum) carries a non-finite loss of any rank to every rank, as it carries a non-finite gradient;
+ *   all-reduce(sum) of the n + 1 floats;
+ *   gj_nonfinite_check    : one launch (one CTA), skip[0] = 1 if any of x[0..n) is not finite, else 0; flag (may be NULL) receives the
+ *                           same decision as 1.f / 0.f (the trainer's stats slot 6).  Every rank reads the same buffer, so every rank
+ *                           takes the same decision;
+ *   gj_adam_step_flat_guarded / gj_optimizer_step_flat_guarded: gj_adam_step_flat / gj_optimizer_step_flat that return without
+ *                           writing anything when skip[0] != 0.  step_state (2 int32, zero-initialised by the caller): step_state[0]
+ *                           counts the updates applied, and the guarded Adam takes step_state[0] + 1 as its 1-based step (the bias
+ *                           corrections count applied updates only); the last CTA of an applied update advances it.  step_state[1] is
+ *                           the kernels' arrival counter, left at 0 by every launch.  step_state may be NULL for the guarded
+ *                           RMSprop / Adagrad / SGD (nothing counted).  Updates that are applied equal the unguarded kernels' bit for bit.
+ * All four are capturable in a CUDA graph and allocate nothing. */
+int gj_nonfinite_flag(const float* terms, int32_t count, float* out, void* stream);
+int gj_nonfinite_check(const float* x, size_t n, int32_t* skip, float* flag, void* stream);
+int gj_adam_step_flat_guarded(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr, float beta1,
+                              float beta2, float eps, const int32_t* skip, int32_t* step_state, float grad_scale, float l1_lambda,
+                              float l2_lambda, void* stream);
+int gj_optimizer_step_flat_guarded(int32_t kind, float* param, const float* grad, float* momentum_buf, float* sq_acc, size_t n, float lr,
+                                   float alpha, float momentum, float eps, float grad_scale, float l1_lambda, float l2_lambda,
+                                   const int32_t* skip, int32_t* step_state, void* stream);
 
 /* sum|p| and sum p^2 over n floats into out[0], out[1] (overwritten; deterministic two-stage). */
 int gj_param_norms(const float* param, size_t n, float* out, void* workspace, size_t workspace_bytes, void* stream);
