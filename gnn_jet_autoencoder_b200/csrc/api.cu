@@ -4,6 +4,8 @@
 #include <stdio.h>
 #include <stdlib.h>
 
+#include <algorithm>
+
 #include "gj_common.cuh"
 
 static thread_local char g_err[512] = "";
@@ -145,9 +147,56 @@ int32_t gj_set_deterministic(int32_t on) {
   return prev;
 }
 
+// The kernels one message-passing step runs, resolved once per (layout, precision) by step_plan(); every launch sequence,
+// workspace plan and launch count below reads it.  Edge kernels: SIMT (edge_simt.cu), first-generation tcgen05 (edge_tc.cu),
+// the second- and third-generation fused kernels (edge_fwd2.cu / edge_bwd2.cu, edge3.cu), and the edge MLP as generic GEMMs
+// over the materialised edge rows of a chunk of jets (dense.cu).
+enum StepEdge { EDGE_SIMT, EDGE_TC1, EDGE_TC2, EDGE_TC3, EDGE_MAT };
+struct StepPath {
+  int precision;
+  StepEdge edge;
+  bool dense_node;      // the node level (P|Q projections, node MLP and their adjoints) as generic GEMMs (dense.cu)
+  bool post_tc, pre_tc;      // the node-MLP adjoint / the projections' adjoint on tcgen05 (node_tc.cu); EDGE_TC2 only
+  // the backward with both node-level adjoints on tcgen05: their partials and the edge kernel's are reduced together
+  bool tail_fused() const { return post_tc && pre_tc; }
+  // the fused kernels can keep P|Q, the parameter image and the pair distances for the backward (gj_mp_step_saved_bytes)
+  bool saves() const { return edge == EDGE_TC2 || edge == EDGE_TC3; }
+};
+
+static StepPath resolve_path(const MPLayout& L, int precision) {
+  StepPath p = {precision, EDGE_MAT, false, false, false};
+  const bool tc = precision == GJ_PREC_BF16 && L.Le > 1;      // a one-layer edge network runs the SIMT kernels in either mode
+  if (tc && gj_fwd2_supported(L) && gj_bwd2_supported(L)) p.edge = EDGE_TC2;      // forward and backward cover the same widths
+  else if (tc && gj_edge3_supported(L)) p.edge = EDGE_TC3;      // two-layer edge networks [H, H], H = 64 / 128 (BASELINE config 5)
+  else if (tc ? gj_edge_tc_fits(L) : gj_edge_simt_fits(L, nullptr)) p.edge = tc ? EDGE_TC1 : EDGE_SIMT;
+  // else EDGE_MAT: the widths no edge kernel has a plan for (e.g. edge_sizes [[256, 256]])
+  const bool tc2 = p.edge == EDGE_TC2;
+  p.post_tc = tc2 && gj_node_post_bwd_tc_supported(L);
+  p.pre_tc = tc2 && gj_node_pre_bwd_tc_supported(L);
+  // Generic-GEMM node level wherever a node-level weight matrix does not fit the fused node kernels' shared-memory plans, and
+  // for wide layers (BASELINE config 5: H >= 64), where the GEMM formulation -- tcgen05 in the bf16 mode -- is the faster one
+  int wmax = L.H > L.E[0] ? L.H : L.E[0];
+  for (int m = 0; m < L.Ln; ++m) if (L.O[m] > wmax) wmax = L.O[m];
+  p.dense_node = !tc2 && (p.edge == EDGE_MAT || !gj_node_generic_fits(L) || wmax >= 64);
+  return p;
+}
+
+// Validates the descriptor, fills the layout and resolves the step's path.  An entry point that reports errors passes its name
+// (a chain entry point also the step's index) and gets "<who>: <reason>" as the last error; the size queries pass none.
+static int step_plan(const gj_mp_desc* d, MPLayout* L, StepPath* p, const char* who = nullptr, int step = -1) {
+  const char* why;
+  if (int rc = gj_fill_arch(d, L, &why)) {
+    if (who && step >= 0) gj_set_error("%s: %s (step %d)", who, why, step);
+    else if (who) gj_set_error("%s: %s", who, why);
+    return rc;
+  }
+  *p = resolve_path(*L, d->precision);
+  return GJ_OK;
+}
+
 size_t gj_mp_param_count(const gj_mp_desc* d) {
-  MPLayout L; const char* why;
-  if (gj_fill_arch(d, &L, &why)) return 0;
+  MPLayout L; StepPath p;
+  if (step_plan(d, &L, &p)) return 0;
   return (size_t)L.nparams;
 }
 
@@ -156,42 +205,6 @@ static size_t align_floats(size_t n) { return (n + 63) & ~(size_t)63; }   // kee
 struct StepWs {   // offsets in floats
   size_t pq, dpq, de, part, part_post, part_pre, epart, wimg, dist, ysave, dense, emat, total;
 };
-
-static bool use_tc(const MPLayout& L, int precision) { return precision == GJ_PREC_BF16 && L.Le > 1; }
-// the step runs the second-generation fused kernels (forward and backward are covered by the same widths)
-static bool tc2_path(const MPLayout& L, int precision) {
-  return use_tc(L, precision) && gj_fwd2_supported(L) && gj_bwd2_supported(L);
-}
-
-static bool edge_mat(const MPLayout& L, int precision);
-// the step runs the third-generation fused kernels (two-layer edge networks [H, H], H = 64 / 128: BASELINE config 5)
-static bool tc3_path(const MPLayout& L, int precision) {
-  return use_tc(L, precision) && !tc2_path(L, precision) && gj_edge3_supported(L);
-}
-
-// Node-level work (P|Q projections, node MLP and their adjoints) as generic GEMMs (dense.cu): wherever a node-level weight
-// matrix does not fit the fused node kernels' shared-memory plans, and for wide layers (BASELINE config 5: H >= 64), where the
-// GEMM formulation -- tcgen05 in the bf16 mode -- is the faster one
-static bool dense_node(const MPLayout& L, int precision) {
-  if (edge_mat(L, precision)) return true;
-  if (tc2_path(L, precision)) return false;
-  if (!gj_node_generic_fits(L)) return true;
-  int wmax = L.H > L.E[0] ? L.H : L.E[0];
-  for (int m = 0; m < L.Ln; ++m) if (L.O[m] > wmax) wmax = L.O[m];
-  return wmax >= 64;
-}
-
-// The edge MLP as generic GEMMs over the materialised edge rows of a chunk of jets (dense.cu): for the widths no fused edge
-// kernel has a plan for (e.g. edge_sizes [[256, 256]])
-static bool edge_mat(const MPLayout& L, int precision) {
-  if (tc2_path(L, precision) || tc3_path(L, precision)) return false;
-  return use_tc(L, precision) ? !gj_edge_tc_fits(L) : !gj_edge_simt_fits(L, nullptr);
-}
-
-// backward of the bf16 step with both node-level adjoints on tcgen05: their partials and the edge kernel's are reduced together
-static bool node_tail_fused(const MPLayout& L, int precision) {
-  return tc2_path(L, precision) && gj_node_post_bwd_tc_supported(L) && gj_node_pre_bwd_tc_supported(L);
-}
 
 // caller-owned buffer of a step whose parameter-gradient reduction is deferred (gj_mp_step_bwd_deferred): per-CTA partials of the
 // edge kernel, the projections' adjoint and the node-MLP adjoint (offsets in floats)
@@ -204,58 +217,84 @@ static PartialsPlan plan_partials(const MPLayout& L) {
   p.total = off;
   return p;
 }
+static bool can_defer(const MPLayout& L, const StepPath& p) { return L.B > 0 && p.tail_fused(); }
 
-static StepWs plan_ws(const MPLayout& L, int precision, bool backward) {
+static StepWs plan_ws(const MPLayout& L, const StepPath& p, bool backward) {
   StepWs w; size_t off = 0;
   const size_t rows = (size_t)L.B * L.N;
   // P|Q, the packed edge-parameter image and the pair distances come first: a caller-owned "saved" buffer of
   // gj_mp_step_saved_bytes() has exactly this prefix layout
   w.pq = off; off += align_floats(rows * 2 * L.E0p);
   w.wimg = w.dist = off;
-  if (tc2_path(L, precision) || tc3_path(L, precision)) {
-    w.wimg = off; off += align_floats(tc3_path(L, precision) ? gj_edge3_wimage_floats(L) : gj_wimage_floats());
+  if (p.saves()) {
+    w.wimg = off; off += align_floats(p.edge == EDGE_TC3 ? gj_edge3_wimage_floats(L) : gj_wimage_floats());
     w.dist = off; off += align_floats(rows * (size_t)(((L.N + 31) / 32) * 32));
   }
   w.ysave = off;
-  if (tc3_path(L, precision)) off += align_floats(gj_dense_ysave_floats(L));      // node-MLP activations (the saved prefix ends here)
+  if (p.edge == EDGE_TC3) off += align_floats(gj_dense_ysave_floats(L));      // node-MLP activations (the saved prefix ends here)
   w.epart = off;
-  if (!backward && tc2_path(L, precision)) off += align_floats(gj_fwd2_ws_floats(L));   // per-j-block partial aggregates (N > 32)
-  if (!backward && tc3_path(L, precision)) off += align_floats(gj_edge3_fwd_ws_floats(L));
+  if (!backward && p.edge == EDGE_TC2) off += align_floats(gj_fwd2_ws_floats(L));   // per-j-block partial aggregates (N > 32)
+  if (!backward && p.edge == EDGE_TC3) off += align_floats(gj_edge3_fwd_ws_floats(L));
   w.dpq = w.de = w.part = off;
   if (backward) {
     w.dpq = off; off += align_floats(rows * 2 * L.E0p);
     w.de = off; off += align_floats(rows * L.EL);
-    size_t p = gj_node_post_bwd_ws_floats(L);
-    if (tc2_path(L, precision) && gj_node_post_bwd_tc_supported(L)) { const size_t p2 = gj_node_post_bwd_tc_ws_floats(L); if (p2 > p) p = p2; }
-    size_t q = gj_node_pre_bwd_ws_floats(L);
-    if (tc2_path(L, precision) && gj_node_pre_bwd_tc_supported(L)) { const size_t q2 = gj_node_pre_bwd_tc_ws_floats(L); if (q2 > q) q = q2; }
-    size_t r = use_tc(L, precision) ? gj_edge_bwd_tc_ws_floats(L) : (size_t)gj_edge_grid(L.B) * L.pV[0];
-    if (tc2_path(L, precision)) { const size_t r2 = gj_bwd2_ws_floats(L); if (r2 > r) r = r2; }
-    if (tc3_path(L, precision)) { const size_t r2 = gj_edge3_bwd_ws_floats(L); if (r2 > r) r = r2; }
-    if (q > p) p = q;
-    if (r > p) p = r;
-    if (p < 64) p = 64;
-    w.part = off; off += align_floats(p);
+    // per-CTA parameter-gradient partials of the node-level and edge adjoints, which use the region one after another.  The fused
+    // node kernels' and the first-generation edge adjoint's sizes count on every path (the latter also covers the SIMT adjoint)
+    size_t n = std::max({gj_node_post_bwd_ws_floats(L), gj_node_pre_bwd_ws_floats(L), gj_edge_bwd_tc_ws_floats(L), (size_t)64});
+    if (p.post_tc) n = std::max(n, gj_node_post_bwd_tc_ws_floats(L));
+    if (p.pre_tc) n = std::max(n, gj_node_pre_bwd_tc_ws_floats(L));
+    if (p.edge == EDGE_TC2) n = std::max(n, gj_bwd2_ws_floats(L));
+    if (p.edge == EDGE_TC3) n = std::max(n, gj_edge3_bwd_ws_floats(L));
+    w.part = off; off += align_floats(n);
     // the all-tensor-core backward keeps the node-MLP and projection partials next to the edge kernel's, so that one
     // launch reduces all three at the end of the step
     w.part_post = w.part_pre = w.part;
-    if (node_tail_fused(L, precision)) {
+    if (p.tail_fused()) {
       w.part_post = off; off += align_floats(gj_node_post_bwd_tc_ws_floats(L));
       w.part_pre = off; off += align_floats(gj_node_pre_bwd_tc_ws_floats(L));
     }
   }
   w.dense = off;
-  if (dense_node(L, precision)) off += align_floats(gj_dense_ws_floats(L, backward));
+  if (p.dense_node) off += align_floats(gj_dense_ws_floats(L, backward));
   w.emat = off;
-  if (edge_mat(L, precision)) off += align_floats(gj_edge_mat_ws_floats(L, backward));
+  if (p.edge == EDGE_MAT) off += align_floats(gj_edge_mat_ws_floats(L, backward));
   w.total = off;
   return w;
 }
 
+// The step's edge kernel, forward: e from h and P|Q.  `pre` is the caller's saved buffer or the workspace (same layout).
+static int edge_fwd(const MPLayout& L, const StepPath& p, const StepWs& w, float* ws, float* pre, bool saved, bool prepacked,
+                    const float* h, const float* params, float* e_out, cudaStream_t st) {
+  switch (p.edge) {
+    case EDGE_SIMT: return gj_edge_fwd_simt(L, h, pre + w.pq, params, e_out, st);
+    case EDGE_TC1: return gj_edge_fwd_tc(L, h, pre + w.pq, params, e_out, st);
+    case EDGE_TC2: return gj_edge_fwd2(L, h, pre + w.pq, params, e_out, ws + w.epart, pre + w.wimg, saved ? pre + w.dist : nullptr, st, false, prepacked);
+    case EDGE_TC3: return gj_edge_fwd3(L, h, pre + w.pq, params, e_out, ws + w.epart, pre + w.wimg, pre + w.dist, st);
+    case EDGE_MAT: break;
+  }
+  return gj_edge_mat_fwd(L, h, pre + w.pq, params, e_out, ws + w.emat, p.precision, st);
+}
+
+// The step's edge adjoint: dP|dQ, the distance-path dh and the edge parameter gradients from de
+static int edge_bwd(const MPLayout& L, const StepPath& p, const StepWs& w, float* ws, float* pre, bool saved, const float* h,
+                    const float* params, float* dh, float* dparams, cudaStream_t st) {
+  switch (p.edge) {
+    case EDGE_SIMT: return gj_edge_bwd_simt(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, st);
+    case EDGE_TC1: return gj_edge_bwd_tc(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, st);
+    case EDGE_TC2:
+      return gj_edge_bwd2(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, pre + w.wimg, pre + w.dist, saved,
+                          st, 0, nullptr, nullptr, nullptr);
+    case EDGE_TC3: return gj_edge_bwd3(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, pre + w.wimg, pre + w.dist, saved, st);
+    case EDGE_MAT: break;
+  }
+  return gj_edge_mat_bwd(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.emat, p.precision, st);
+}
+
 size_t gj_mp_step_fwd_workspace(const gj_mp_desc* d) {
-  MPLayout L; const char* why;
-  if (gj_fill_arch(d, &L, &why)) return 0;
-  return plan_ws(L, d->precision, false).total * sizeof(float);
+  MPLayout L; StepPath p;
+  if (step_plan(d, &L, &p)) return 0;
+  return plan_ws(L, p, false).total * sizeof(float);
 }
 
 // saved: optional caller-owned buffer of gj_mp_step_saved_bytes(): receives P|Q, the packed edge parameters and the pair
@@ -265,29 +304,21 @@ static int mp_step_fwd_impl(const gj_mp_desc* d, const float* h, const float* pa
   g_err[0] = 0;
   if (!d || !h || !params || !h_out || !e_out || !workspace) { gj_set_error("%s: null pointer", who); return GJ_ERR_INVALID; }
   if (d->precision != GJ_PREC_FP32 && d->precision != GJ_PREC_BF16) { gj_set_error("%s: unknown precision %d", who, d->precision); return GJ_ERR_INVALID; }
-  MPLayout L; const char* why;
-  int rc = gj_fill_arch(d, &L, &why);
-  if (rc) { gj_set_error("%s: %s", who, why); return rc; }
+  MPLayout L; StepPath p;
+  int rc = step_plan(d, &L, &p, who);
+  if (rc) return rc;
   if (L.B == 0) return GJ_OK;
-  const StepWs w = plan_ws(L, d->precision, false);
+  const StepWs w = plan_ws(L, p, false);
   if (workspace_bytes < w.total * sizeof(float)) { gj_set_error("%s: workspace too small", who); return GJ_ERR_WORKSPACE; }
   float* ws = (float*)workspace;
-  const bool emat = edge_mat(L, d->precision);
-  const bool tc2 = tc2_path(L, d->precision);
-  const bool tc3 = tc3_path(L, d->precision);
-  if (saved && !tc2 && !tc3) { gj_set_error("%s: this step has nothing to save (gj_mp_step_saved_bytes is 0)", who); return GJ_ERR_INVALID; }
-  if (prepacked && !(tc2 && saved)) { gj_set_error("%s: this step has no packed parameter image (gj_mp_step_partials_bytes is 0)", who); return GJ_ERR_INVALID; }
+  if (saved && !p.saves()) { gj_set_error("%s: this step has nothing to save (gj_mp_step_saved_bytes is 0)", who); return GJ_ERR_INVALID; }
+  if (prepacked && !(p.edge == EDGE_TC2 && saved)) {
+    gj_set_error("%s: this step has no packed parameter image (gj_mp_step_partials_bytes is 0)", who); return GJ_ERR_INVALID; }
   float* pre = saved ? (float*)saved : ws;      // P|Q, parameter image, pair distances: same layout in either buffer
   cudaStream_t st = (cudaStream_t)stream;
-  const bool dense = dense_node(L, d->precision);
-  if ((rc = dense ? gj_dense_pre_fwd(L, h, params, pre + w.pq, d->precision, st) : gj_node_pre_fwd(L, h, params, pre + w.pq, st))) return rc;
-  if (emat) rc = gj_edge_mat_fwd(L, h, ws + w.pq, params, e_out, ws + w.emat, d->precision, st);
-  else if (tc3) rc = gj_edge_fwd3(L, h, pre + w.pq, params, e_out, ws + w.epart, pre + w.wimg, pre + w.dist, st);
-  else if (tc2) rc = gj_edge_fwd2(L, h, pre + w.pq, params, e_out, ws + w.epart, pre + w.wimg, saved ? pre + w.dist : nullptr, st, false, prepacked);
-  else rc = use_tc(L, d->precision) ? gj_edge_fwd_tc(L, h, ws + w.pq, params, e_out, st)
-                                    : gj_edge_fwd_simt(L, h, ws + w.pq, params, e_out, st);
-  if (rc) return rc;
-  if (dense) return gj_dense_post_fwd(L, e_out, h, params, h_out, ws + w.dense, (saved && tc3) ? pre + w.ysave : nullptr, d->precision, st);
+  if ((rc = p.dense_node ? gj_dense_pre_fwd(L, h, params, pre + w.pq, d->precision, st) : gj_node_pre_fwd(L, h, params, pre + w.pq, st))) return rc;
+  if ((rc = edge_fwd(L, p, w, ws, pre, saved != nullptr, prepacked, h, params, e_out, st))) return rc;
+  if (p.dense_node) return gj_dense_post_fwd(L, e_out, h, params, h_out, ws + w.dense, (saved && p.edge == EDGE_TC3) ? pre + w.ysave : nullptr, d->precision, st);
   return gj_node_post_fwd(L, e_out, h, params, h_out, st);
 }
 
@@ -297,27 +328,27 @@ int gj_mp_step_fwd(const gj_mp_desc* d, const float* h, const float* params, flo
 }
 
 int gj_mp_step_launches(const gj_mp_desc* d, int backward, int with_saved) {
-  MPLayout L; const char* why;
-  if (gj_fill_arch(d, &L, &why)) return 0;
-  const bool tc2 = tc2_path(L, d->precision);
-  const int njb = (tc2 && L.N > 32) ? 1 : 0;      // per-j-block partial sums (forward: e, backward: dP)
-  if (edge_mat(L, d->precision)) return gj_dense_launches(L, backward != 0) + gj_edge_mat_launches(L, backward != 0);
-  if (tc3_path(L, d->precision))      // + parameter image, pair distances, edge kernel [, j-block sum]; backward also the distance adjoint and the reduction
-    return gj_dense_launches(L, backward != 0) + 3 + (L.N > 32 ? 1 : 0) + (backward ? 2 : 0) - ((backward && with_saved) ? 4 + L.Ln + 1 : 0);
-  if (dense_node(L, d->precision)) return gj_dense_launches(L, backward != 0) + (backward ? 2 : 1);      // + the edge kernel(s)
-  if (!backward) return tc2 ? 4 + njb : 3;        // projections, [parameter image], edge kernel, [j-block sum], node MLP
-  if (!tc2) return 8;
+  MPLayout L; StepPath p;
+  if (step_plan(d, &L, &p)) return 0;
+  const int njb = L.N > 32 ? 1 : 0;      // the fused kernels' per-j-block partial sums (forward: e, backward: dP)
+  if (p.dense_node) {
+    const int node = gj_dense_launches(L, backward != 0);
+    if (p.edge == EDGE_MAT) return node + gj_edge_mat_launches(L, backward != 0);
+    if (p.edge == EDGE_TC3)      // + parameter image, pair distances, edge kernel [, j-block sum]; backward also the distance adjoint and the reduction
+      return node + 3 + njb + (backward ? 2 : 0) - ((backward && with_saved) ? 4 + L.Ln + 1 : 0);
+    return node + (backward ? 2 : 1);      // + the edge kernel(s)
+  }
+  if (!backward) return p.edge == EDGE_TC2 ? 4 + njb : 3;      // projections, [parameter image], edge kernel, [j-block sum], node MLP
+  if (p.edge != EDGE_TC2) return 8;
   // node MLP adjoint, [projections, parameter image, pair distances unless saved], edge kernel, [dP j-block sum],
   // pair-distance adjoint, projections' adjoint, and one reduction (all-tensor-core tail) or three
-  const int reductions = node_tail_fused(L, d->precision) ? 1 : 3;
-  return 4 + reductions + njb + ((with_saved && tc2) ? 0 : 3);
+  return 4 + (p.tail_fused() ? 1 : 3) + njb + (with_saved ? 0 : 3);
 }
 
 size_t gj_mp_step_saved_bytes(const gj_mp_desc* d) {
-  MPLayout L; const char* why;
-  if (gj_fill_arch(d, &L, &why) || !(tc2_path(L, d->precision) || tc3_path(L, d->precision))) return 0;
-  const StepWs w = plan_ws(L, d->precision, false);
-  return w.epart * sizeof(float);      // the prefix P|Q, parameter image, pair distances
+  MPLayout L; StepPath p;
+  if (step_plan(d, &L, &p) || !p.saves()) return 0;
+  return plan_ws(L, p, false).epart * sizeof(float);      // the prefix P|Q, parameter image, pair distances
 }
 
 int gj_mp_step_fwd_saving(const gj_mp_desc* d, const float* h, const float* params, float* h_out, float* e_out, void* saved,
@@ -327,9 +358,9 @@ int gj_mp_step_fwd_saving(const gj_mp_desc* d, const float* h, const float* para
 }
 
 size_t gj_mp_step_bwd_workspace(const gj_mp_desc* d) {
-  MPLayout L; const char* why;
-  if (gj_fill_arch(d, &L, &why)) return 0;
-  return plan_ws(L, d->precision, true).total * sizeof(float);
+  MPLayout L; StepPath p;
+  if (step_plan(d, &L, &p)) return 0;
+  return plan_ws(L, p, true).total * sizeof(float);
 }
 
 // partials (optional, with saved): caller-owned buffer of gj_mp_step_partials_bytes(); the per-CTA parameter-gradient partials are
@@ -340,23 +371,20 @@ static int mp_step_bwd_impl(const gj_mp_desc* d, const float* h, const float* e,
   g_err[0] = 0;
   if (!d || !h || !e || !params || !dh_out || !dh || (!dparams && !partials) || !workspace) { gj_set_error("%s: null pointer", who); return GJ_ERR_INVALID; }
   if (d->precision != GJ_PREC_FP32 && d->precision != GJ_PREC_BF16) { gj_set_error("%s: unknown precision %d", who, d->precision); return GJ_ERR_INVALID; }
-  MPLayout L; const char* why;
-  int rc = gj_fill_arch(d, &L, &why);
-  if (rc) { gj_set_error("%s: %s", who, why); return rc; }
+  MPLayout L; StepPath p;
+  int rc = step_plan(d, &L, &p, who);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   if (L.B == 0 && partials) { gj_set_error("%s: empty batch", who); return GJ_ERR_INVALID; }
   if (L.B == 0) { cudaMemsetAsync(dparams, 0, (size_t)L.nparams * sizeof(float), st); return GJ_OK; }
-  const StepWs w = plan_ws(L, d->precision, true);
+  const StepWs w = plan_ws(L, p, true);
   if (workspace_bytes < w.total * sizeof(float)) { gj_set_error("%s: workspace too small", who); return GJ_ERR_WORKSPACE; }
   float* ws = (float*)workspace;
-  const bool emat = edge_mat(L, d->precision);
-  const bool tc2 = tc2_path(L, d->precision);
-  const bool tc3 = tc3_path(L, d->precision);
-  if (saved && !tc2 && !tc3) { gj_set_error("%s: this step has nothing saved (gj_mp_step_saved_bytes is 0)", who); return GJ_ERR_INVALID; }
+  if (saved && !p.saves()) { gj_set_error("%s: this step has nothing saved (gj_mp_step_saved_bytes is 0)", who); return GJ_ERR_INVALID; }
   float* pre = saved ? (float*)saved : ws;      // read-only when it is the caller's saved buffer
-  if (partials && !(node_tail_fused(L, d->precision) && saved)) {
+  if (partials && !(p.tail_fused() && saved)) {
     gj_set_error("%s: this step cannot defer its reduction (gj_mp_step_partials_bytes is 0)", who); return GJ_ERR_INVALID; }
-  if (node_tail_fused(L, d->precision)) {
+  if (p.tail_fused()) {
     // node MLP adjoint (also clears dP|dQ), P|Q unless saved, edge adjoint, projections' adjoint, one reduction of all partials
     int np_post = 0, np_pre = 0, np_edge = 0;
     const float* part_edge = nullptr;
@@ -372,36 +400,24 @@ static int mp_step_bwd_impl(const gj_mp_desc* d, const float* h, const float* e,
     if (partials) return GJ_OK;      // reduced later, together with the other steps' (gj_mp_steps_reduce)
     return gj_reduce_step_partials(L, part_edge, np_edge, part_pre, np_pre, part_post, np_post, dparams, st);
   }
-  const bool dense = dense_node(L, d->precision);
-  if (dense) {      // generic-GEMM node level (dense.cu) around the edge adjoint
-    if ((rc = gj_dense_post_bwd(L, e, h, params, dh_out, ws + w.de, dh, dparams, ws + w.dense, (saved && tc3) ? pre + w.ysave : nullptr,
-                                d->precision, st))) return rc;
+  if (p.dense_node) {      // generic-GEMM node level (dense.cu) around the edge adjoint
+    if ((rc = gj_dense_post_bwd(L, e, h, params, dh_out, ws + w.de, dh, dparams, ws + w.dense,
+                                (saved && p.edge == EDGE_TC3) ? pre + w.ysave : nullptr, d->precision, st))) return rc;
     if (!saved && (rc = gj_dense_pre_fwd(L, h, params, pre + w.pq, d->precision, st))) return rc;
-    rc = emat ? gj_edge_mat_bwd(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.emat, d->precision, st)
-       : tc3 ? gj_edge_bwd3(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, pre + w.wimg, pre + w.dist,
-                            saved != nullptr, st)
-       : use_tc(L, d->precision) ? gj_edge_bwd_tc(L, h, ws + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, st)
-                                 : gj_edge_bwd_simt(L, h, ws + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, st);
-    if (rc) return rc;
+    if ((rc = edge_bwd(L, p, w, ws, pre, saved != nullptr, h, params, dh, dparams, st))) return rc;
     return gj_dense_pre_bwd(L, h, params, ws + w.dpq, dh, dparams, ws + w.dense, d->precision, st);
   }
   // node MLP adjoint: de, node-path dh, node parameter gradients
-  if (tc2 && gj_node_post_bwd_tc_supported(L)) {      // bf16 mode: the node MLP adjoint on tcgen05
+  if (p.post_tc) {      // bf16 mode: the node MLP adjoint on tcgen05
     int nparts = 0;
     if ((rc = gj_node_post_bwd_tc(L, e, h, params, dh_out, ws + w.de, dh, ws + w.part, &nparts, nullptr, st))) return rc;
     if ((rc = gj_reduce_partials(ws + w.part, nparts, L.nparams - L.pV[0], dparams + L.pV[0], st))) return rc;
   } else if ((rc = gj_node_post_bwd(L, e, h, params, dh_out, ws + w.de, dh, dparams, ws + w.part, st))) return rc;
-  // P|Q (recomputed unless saved by the forward call), then the edge adjoint: dP|dQ, distance-path dh, edge parameter gradients
+  // P|Q (recomputed unless saved by the forward call), then the edge adjoint
   if (!saved && (rc = gj_node_pre_fwd(L, h, params, pre + w.pq, st))) return rc;
-  if (tc2)
-    rc = gj_edge_bwd2(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, pre + w.wimg, pre + w.dist, saved != nullptr,
-                      st, 0, nullptr, nullptr, nullptr);
-  else
-    rc = use_tc(L, d->precision) ? gj_edge_bwd_tc(L, h, ws + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, st)
-                                 : gj_edge_bwd_simt(L, h, ws + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, st);
-  if (rc) return rc;
+  if ((rc = edge_bwd(L, p, w, ws, pre, saved != nullptr, h, params, dh, dparams, st))) return rc;
   // first-layer projections' adjoint: dh += Wa^T dP + Wb^T dQ, dWa, dWb, db0
-  if (tc2 && gj_node_pre_bwd_tc_supported(L)) {      // bf16 mode: the projections' adjoint on tcgen05
+  if (p.pre_tc) {      // bf16 mode: the projections' adjoint on tcgen05
     int nparts = 0;
     if ((rc = gj_node_pre_bwd_tc(L, h, params, ws + w.dpq, dh, ws + w.part, &nparts, st))) return rc;
     return gj_reduce_pre_partials(L, ws + w.part, nparts, dparams, st);
@@ -422,8 +438,8 @@ int gj_mp_step_bwd_saved(const gj_mp_desc* d, const float* h, const float* e, co
 
 // ---- a chain of steps: ONE launch packs every step's parameter image, ONE launch reduces every step's gradient partials ----
 size_t gj_mp_step_partials_bytes(const gj_mp_desc* d) {
-  MPLayout L; const char* why;
-  if (gj_fill_arch(d, &L, &why) || L.B == 0 || !node_tail_fused(L, d->precision)) return 0;
+  MPLayout L; StepPath p;
+  if (step_plan(d, &L, &p) || !can_defer(L, p)) return 0;
   return plan_partials(L).total * sizeof(float);
 }
 
@@ -432,12 +448,12 @@ int gj_mp_steps_pack(int32_t n, const gj_mp_desc* const* descs, const float* con
   if (n < 0 || n > 64 || (n > 0 && (!descs || !params || !saved))) { gj_set_error("gj_mp_steps_pack: bad arguments"); return GJ_ERR_INVALID; }
   MPLayout Ls[64]; float* img[64];
   for (int s = 0; s < n; ++s) {
-    const char* why;
+    StepPath p;
     if (!descs[s] || !params[s] || !saved[s]) { gj_set_error("gj_mp_steps_pack: null pointer (step %d)", s); return GJ_ERR_INVALID; }
-    if (int rc = gj_fill_arch(descs[s], &Ls[s], &why)) { gj_set_error("gj_mp_steps_pack: %s (step %d)", why, s); return rc; }
-    if (gj_mp_step_partials_bytes(descs[s]) == 0) {
+    if (int rc = step_plan(descs[s], &Ls[s], &p, "gj_mp_steps_pack", s)) return rc;
+    if (!can_defer(Ls[s], p)) {
       gj_set_error("gj_mp_steps_pack: step %d does not run the fused tensor-core kernels (gj_mp_step_partials_bytes is 0)", s); return GJ_ERR_INVALID; }
-    img[s] = (float*)saved[s] + plan_ws(Ls[s], descs[s]->precision, false).wimg;
+    img[s] = (float*)saved[s] + plan_ws(Ls[s], p, false).wimg;
   }
   return n ? gj_pack_batch2(n, Ls, params, img, (cudaStream_t)stream) : GJ_OK;
 }
@@ -462,10 +478,10 @@ int gj_mp_steps_reduce(int32_t n, const gj_mp_desc* const* descs, const void* co
   const float* pE[64]; const float* pP[64]; const float* pN[64];
   int nE[64], nP[64], nN[64];
   for (int s = 0; s < n; ++s) {
-    const char* why;
+    StepPath p;
     if (!descs[s] || !partials[s] || !dparams[s]) { gj_set_error("gj_mp_steps_reduce: null pointer (step %d)", s); return GJ_ERR_INVALID; }
-    if (int rc = gj_fill_arch(descs[s], &Ls[s], &why)) { gj_set_error("gj_mp_steps_reduce: %s (step %d)", why, s); return rc; }
-    if (gj_mp_step_partials_bytes(descs[s]) == 0) {
+    if (int rc = step_plan(descs[s], &Ls[s], &p, "gj_mp_steps_reduce", s)) return rc;
+    if (!can_defer(Ls[s], p)) {
       gj_set_error("gj_mp_steps_reduce: step %d cannot defer its reduction (gj_mp_step_partials_bytes is 0)", s); return GJ_ERR_INVALID; }
     const PartialsPlan pp = plan_partials(Ls[s]);
     const float* base = (const float*)partials[s];
@@ -659,28 +675,29 @@ int gj_mse_fwd_bwd(size_t count, double denom, const float* p, const float* q, f
 
 /* Measurement hooks (declared in the header under "benchmark support"): relaunch ONLY the fused edge kernel of a step on
  * the workspace that a preceding full gj_mp_step_fwd / gj_mp_step_bwd call with the same arguments has populated. */
+static int bench_step(const gj_mp_desc* d, bool pointers, size_t workspace_bytes, bool backward, const char* who, MPLayout* L, StepWs* w) {
+  g_err[0] = 0;
+  StepPath p;
+  if (int rc = step_plan(d, L, &p, who)) return rc;
+  if (!pointers) { gj_set_error("%s: null pointer", who); return GJ_ERR_INVALID; }
+  if (p.edge != EDGE_TC2) { gj_set_error("%s: step does not run the fused tensor-core kernel", who); return GJ_ERR_INVALID; }
+  *w = plan_ws(*L, p, backward);
+  if (workspace_bytes < w->total * sizeof(float)) { gj_set_error("%s: workspace too small", who); return GJ_ERR_WORKSPACE; }
+  return GJ_OK;
+}
+
 int gj_bench_edge_fwd_only(const gj_mp_desc* d, const float* h, const float* params, float* e_out, void* workspace,
                            size_t workspace_bytes, void* stream) {
-  g_err[0] = 0;
-  MPLayout L; const char* why;
-  int rc = gj_fill_arch(d, &L, &why);
-  if (rc || !h || !params || !e_out || !workspace) { gj_set_error("gj_bench_edge_fwd_only: %s", rc ? why : "null pointer"); return GJ_ERR_INVALID; }
-  if (!tc2_path(L, d->precision)) { gj_set_error("gj_bench_edge_fwd_only: step does not run the fused tensor-core kernel"); return GJ_ERR_INVALID; }
-  const StepWs w = plan_ws(L, d->precision, false);
-  if (workspace_bytes < w.total * sizeof(float)) { gj_set_error("gj_bench_edge_fwd_only: workspace too small"); return GJ_ERR_WORKSPACE; }
+  MPLayout L; StepWs w;
+  if (int rc = bench_step(d, h && params && e_out && workspace, workspace_bytes, false, "gj_bench_edge_fwd_only", &L, &w)) return rc;
   float* ws = (float*)workspace;
   return gj_edge_fwd2(L, h, ws + w.pq, params, e_out, ws + w.epart, ws + w.wimg, nullptr, (cudaStream_t)stream, true, false);
 }
 
 int gj_bench_edge_bwd_only(const gj_mp_desc* d, const float* h, const float* params, float* dh, float* dparams, void* workspace,
                            size_t workspace_bytes, void* stream) {
-  g_err[0] = 0;
-  MPLayout L; const char* why;
-  int rc = gj_fill_arch(d, &L, &why);
-  if (rc || !h || !params || !dh || !dparams || !workspace) { gj_set_error("gj_bench_edge_bwd_only: %s", rc ? why : "null pointer"); return GJ_ERR_INVALID; }
-  if (!tc2_path(L, d->precision)) { gj_set_error("gj_bench_edge_bwd_only: step does not run the fused tensor-core kernel"); return GJ_ERR_INVALID; }
-  const StepWs w = plan_ws(L, d->precision, true);
-  if (workspace_bytes < w.total * sizeof(float)) { gj_set_error("gj_bench_edge_bwd_only: workspace too small"); return GJ_ERR_WORKSPACE; }
+  MPLayout L; StepWs w;
+  if (int rc = bench_step(d, h && params && dh && dparams && workspace, workspace_bytes, true, "gj_bench_edge_bwd_only", &L, &w)) return rc;
   float* ws = (float*)workspace;
   return gj_edge_bwd2(L, h, ws + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, ws + w.wimg, ws + w.dist, true,
                       (cudaStream_t)stream, 1, nullptr, nullptr, nullptr);
@@ -690,13 +707,9 @@ int gj_bench_edge_bwd_only(const gj_mp_desc* d, const float* h, const float* par
  * by the gj_mp_step_bwd_saved call that followed. */
 int gj_bench_edge_bwd_saved_only(const gj_mp_desc* d, const float* h, const float* params, float* dh, float* dparams, const void* saved,
                                  void* workspace, size_t workspace_bytes, void* stream) {
-  g_err[0] = 0;
-  MPLayout L; const char* why;
-  int rc = gj_fill_arch(d, &L, &why);
-  if (rc || !h || !params || !dh || !dparams || !saved || !workspace) { gj_set_error("gj_bench_edge_bwd_saved_only: %s", rc ? why : "null pointer"); return GJ_ERR_INVALID; }
-  if (!tc2_path(L, d->precision)) { gj_set_error("gj_bench_edge_bwd_saved_only: step does not run the fused tensor-core kernel"); return GJ_ERR_INVALID; }
-  const StepWs w = plan_ws(L, d->precision, true);
-  if (workspace_bytes < w.total * sizeof(float)) { gj_set_error("gj_bench_edge_bwd_saved_only: workspace too small"); return GJ_ERR_WORKSPACE; }
+  MPLayout L; StepWs w;
+  if (int rc = bench_step(d, h && params && dh && dparams && saved && workspace, workspace_bytes, true, "gj_bench_edge_bwd_saved_only", &L, &w))
+    return rc;
   float* ws = (float*)workspace;
   float* pre = (float*)saved;
   return gj_edge_bwd2(L, h, pre + w.pq, params, ws + w.de, ws + w.dpq, dh, dparams, ws + w.part, pre + w.wimg, pre + w.dist, true,
@@ -705,13 +718,12 @@ int gj_bench_edge_bwd_saved_only(const gj_mp_desc* d, const float* h, const floa
 
 int gj_mp_plan_info(const gj_mp_desc* d, int32_t* info) {
   g_err[0] = 0;
-  MPLayout L; const char* why;
-  int rc = gj_fill_arch(d, &L, &why);
-  if (rc || !info) { gj_set_error("gj_mp_plan_info: %s", rc ? why : "null pointer"); return GJ_ERR_INVALID; }
+  MPLayout L; StepPath p;
+  if (int rc = step_plan(d, &L, &p, "gj_mp_plan_info")) return rc;
+  if (!info) { gj_set_error("gj_mp_plan_info: null pointer"); return GJ_ERR_INVALID; }
   gj_tc_plan_info(L, info);
-  {      // the second-generation kernels take over where their widths are compiled in
-    if (tc2_path(L, d->precision)) { gj_fwd2_plan(L, info + 0, info + 1); gj_bwd2_plan(L, info + 2, info + 3); }
-  }
+  // the second-generation kernels take over where their widths are compiled in
+  if (p.edge == EDGE_TC2) { gj_fwd2_plan(L, info + 0, info + 1); gj_bwd2_plan(L, info + 2, info + 3); }
   return GJ_OK;
 }
 

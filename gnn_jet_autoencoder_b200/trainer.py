@@ -13,6 +13,7 @@ two Adams) as a fixed sequence of fused kernels over flat buffers.
 """
 from __future__ import annotations
 
+import gc
 from collections import OrderedDict
 from typing import Optional
 
@@ -611,6 +612,9 @@ class GNNAETrainer:
             self._fwd_bwd()                      # eager warm-up: loads the kernels outside the capture
             self.launches_per_step = ops.LAUNCHES["count"] - before + self._apply_launches   # + the optimiser (and the decision)
             torch.cuda.synchronize()
+            # collect dead objects now, not inside the capture: a CUDA graph destroyed there (a dead trainer's, held by a reference
+            # cycle) makes calls that this thread may not make while it captures, and they invalidate the capture
+            gc.collect()
             g = torch.cuda.CUDAGraph()
             # thread-local capture mode: other threads of the process (NCCL's watchdog, a pinned-memory loader) may call into the CUDA
             # runtime while the step is being captured; in the default global mode such a call invalidates a long capture
